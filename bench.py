@@ -2,6 +2,7 @@
 """bench.py — HSD node-pairs/sec for the degree-mode 3-hop distance matrix.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--workload c2|c3|NODESxHOPS]
+                    [--dump-outputs DIR]
 
 One "step" = one full pass of the hot path over the workload graph: k-hop rings
 (bitmap dynamic programming over all nodes, or one frontier BFS per source) -> per-ring degree CDF signatures -> (N>1: one NCCL all-gather of
@@ -9,7 +10,7 @@ the signature table, or peer-memory stores fused into the BFS kernel) -> pairwis
 between signatures) for this rank's share of the symmetric tiles.
 `value` is whole-job unordered node pairs / second with the graph already in HBM;
 `e2e` is the same job through the host-buffer pipeline (pinned host CSR in, pinned
-host float32 matrix out, copies inside the timed region).
+host float32 matrix out, copies inside the timed region).  Both legs time K steps.
 
 Workload (BASELINE.json configs[1]): networkx.barabasi_albert_graph(20000, 5, seed=0),
 3 hops, full N x N.  With N>1 ranks the SAME graph is row-block sharded (strong scaling).
@@ -294,7 +295,8 @@ class Ctx:
 def measure_degree_path(ctx, g, hops, steps, warmup, workload_key):
     """The hot path (rings -> signatures -> [fused all-gather] -> pairwise) on graph `g`, sharded over
     ctx.world ranks: warm-up, then `steps` timed steps (CUDA events, barrier + synchronize on both
-    sides, max over ranks, L2 flushed before every step).  Returns (record, plan, dg)."""
+    sides, max over ranks, L2 flushed before every step).  Returns (record, plan, dg, block): block is this
+    rank's rows of the distance matrix as the last timed step left them."""
     torch = ctx.torch
     from hsd_b200 import engine
     from hsd_b200.sharded import ShardedDegreeHSD
@@ -323,10 +325,10 @@ def measure_degree_path(ctx, g, hops, steps, warmup, workload_key):
             ev[1].record()
         plan.gather()
         if ev is not None:
-            plan.distances(ev[2], ev[3])   # (N > 1: ends with the device-side barrier that completes the blocks)
+            out = plan.distances(ev[2], ev[3])   # (N > 1: ends with the device-side barrier that completes the blocks)
             ev[5].record()
-        else:
-            plan.distances()
+            return out
+        return plan.distances()
 
     for _ in range(max(warmup, 0)):
         one_step()
@@ -341,7 +343,7 @@ def measure_degree_path(ctx, g, hops, steps, warmup, workload_key):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for k in range(steps):
-        one_step(events[k])
+        block = one_step(events[k])
     e1.record()
     torch.cuda.synchronize()
     ctx.barrier()
@@ -451,7 +453,7 @@ def measure_degree_path(ctx, g, hops, steps, warmup, workload_key):
            "launches_per_step": ((2 * hops + 1) if variant == "cols" else
                                  (2 * hops if n <= 32768 or n > 131072 else hops + 2) if variant == "dense"
                                  else (2 if plan.hub_split is not None else 1)) + (2 if plan.n_rows else 1)}
-    return rec, plan, dg
+    return rec, plan, dg, block
 
 
 def workload_config(n, hops, world, peer, n_bins):
@@ -675,7 +677,7 @@ def run_e2e_single(ctx, n, hops, args, pairs):
         model.calculate_structural_distance(0.0, out=host_out)   # synchronises: the result is in host memory
     step()
     api = "model.HSD(graph, name, 0, hop, metric, signal='degree').calculate_structural_distance(0.0, out=pinned)"
-    return _time_e2e(ctx, step, max(3, min(args.steps, 10)), pairs, model._host_pipe, api, host_out)
+    return _time_e2e(ctx, step, args.steps, pairs, model._host_pipe, api, host_out)
 
 
 def run_e2e_sharded(ctx, g, hops, plan, args, pairs):
@@ -686,7 +688,40 @@ def run_e2e_sharded(ctx, g, hops, plan, args, pairs):
     pipe = engine.HostDegreePipeline(g, hops, device=ctx.dev, row0=plan.row0, n_rows=plan.n_rows)
     host_out = torch.empty((pipe.n_rows, g.n), dtype=torch.float32).pin_memory()
     api = "hsd_b200.engine.HostDegreePipeline.run on each rank's row shard (what HSD.calculate_structural_distance(out=) calls)"
-    return _time_e2e(ctx, lambda: pipe.run(host_out), max(3, min(args.steps, 10)), pairs, pipe, api, host_out)
+    return _time_e2e(ctx, lambda: pipe.run(host_out), args.steps, pairs, pipe, api, host_out)
+
+
+DUMP_BYTES = 64 * 1000 * 1000     # --dump-outputs: upper bound on the size of the .npy files together
+
+
+def dump_outputs(ctx, block, row0, n, out_dir):
+    """--dump-outputs: what the timed path computed in its last step, as .npy files in out_dir, so that two
+    builds of the project can be compared output for output (the workload graph is seeded, so the inputs
+    are identical from run to run).  The N x N float32 matrix is too large to store whole; the files are
+      distances_rows.npy      float64 [R]     sampled row ids: numpy default_rng(0), sorted; every row when N is small
+      distances_sample.npy    float32 [R, N]  those rows of the matrix, as computed
+      distances_row_sums.npy  float64 [N]     every row of the matrix summed in float64 (touches the unsampled rows)
+    With N > 1 ranks each rank contributes the rows of its block and rank 0 writes the files."""
+    torch = ctx.torch
+    n_rows = block.shape[0]
+    r = max(1, min(n, (DUMP_BYTES - 8 * n - 4096) // (4 * n + 8)))     # 4096: slack for the three .npy headers
+    rows = np.sort(np.random.default_rng(0).choice(n, size=r, replace=False))
+    sample = torch.zeros((r, n), dtype=torch.float32, device=ctx.dev)
+    sums = torch.zeros(n, dtype=torch.float64, device=ctx.dev)
+    mine = np.nonzero((rows >= row0) & (rows < row0 + n_rows))[0]
+    if mine.size:
+        sample[torch.from_numpy(mine).to(ctx.dev)] = block[torch.from_numpy(rows[mine] - row0).to(ctx.dev)]
+    for c in range(0, n_rows, 4096):
+        end = min(c + 4096, n_rows)
+        sums[row0 + c:row0 + end] = block[c:end].sum(1, dtype=torch.float64)
+    if ctx.world > 1:      # every row is nonzero on exactly one rank
+        ctx.dist.all_reduce(sample)
+        ctx.dist.all_reduce(sums)
+    if ctx.rank == 0:
+        os.makedirs(out_dir, exist_ok=True)
+        np.save(os.path.join(out_dir, "distances_rows.npy"), rows.astype(np.float64))
+        np.save(os.path.join(out_dir, "distances_sample.npy"), sample.cpu().numpy())
+        np.save(os.path.join(out_dir, "distances_row_sums.npy"), sums.cpu().numpy())
 
 
 def run_native(args):
@@ -698,9 +733,12 @@ def run_native(args):
 
     n, hops = parse_workload(args.workload)
     g = powerlaw_graph(n, 5, seed=0)       # same deterministic graph on every rank
-    rec, plan, dg = measure_degree_path(ctx, g, hops, args.steps, args.warmup, args.workload)
+    rec, plan, dg, block = measure_degree_path(ctx, g, hops, args.steps, args.warmup, args.workload)
     peer = rec["peer"]
     pairs = rec["pairs"]
+    if args.dump_outputs:
+        dump_outputs(ctx, block, plan.row0, n, args.dump_outputs)
+    del block
 
     # ---- e2e: host buffers in, host matrix out, copies inside the timed region ----
     # N = 1: literally the call a user of the reference makes — the drop-in class,
@@ -721,7 +759,7 @@ def run_native(args):
         try:
             if key == "c3" and args.workload != "c3":
                 g3 = powerlaw_graph(100000, 5, seed=0)
-                r3, p3, d3 = measure_degree_path(ctx, g3, 4, 3, 1, "c3")
+                r3, p3, d3, _ = measure_degree_path(ctx, g3, 4, 3, 1, "c3")
                 extras["north_star_c3"] = {
                     "config": workload_config(100000, 4, world, r3["peer"], r3["n_bins"]), "n_gpus": world, "steps": 3, "warmup": 1,
                     "ms_per_step": r3["ms_per_step"], "value": r3["value"], "unit": UNIT, "stage_ms": r3["stage_ms"], "stage_ms_per_rank": r3["stage_ms_per_rank"],
@@ -782,7 +820,14 @@ def main():
                     help="other BASELINE.json configs measured after the headline workload, as sub-records of the line")
     ap.add_argument("--no-extras", action="store_true")
     ap.add_argument("--no-e2e", action="store_true", help="skip the host-buffer e2e leg (NVLink byte-count runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write a seeded sample of the distance matrix the last step computed "
+                         "(and its row sums) to DIR/*.npy, at most 64 MB")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the native arm's outputs; the reference arm computes a sample of pairs only")
     if args.impl == "reference":
         run_reference(args)
     else:

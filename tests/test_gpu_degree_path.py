@@ -163,3 +163,35 @@ def test_repeated_sources_fall_back_to_the_frontier_variant(monkeypatch):
     sig, sizes, _, _ = engine.ring_signature_degree(dg, 3, rows=rows)
     ref_sig, ref_sizes, _, _ = engine.ring_signature_degree(dg, 3)
     assert torch.equal(sig, ref_sig[rows.long()]) and torch.equal(sizes, ref_sizes[rows.long()])
+
+
+def test_bench_dump_outputs_hold_the_timed_path_result(tmp_path):
+    """bench.py --dump-outputs: within 64 MB, the seeded sample of rows and the row sums it writes are
+    those of the distance matrix the hot path computes on the same graph; --steps sets the step count."""
+    import json
+    import os
+    import subprocess
+    import sys
+    import torch
+    from hsd_b200 import engine
+    from hsd_b200.graph import powerlaw_graph
+    from hsd_b200.sharded import ShardedDegreeHSD
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    n, hops = 5000, 3                      # the matrix (100 MB) exceeds the dump budget: rows are sampled
+    out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--workload", f"{n}x{hops}", "--steps", "2",
+                          "--warmup", "0", "--no-extras", "--no-cpu-baseline", "--no-e2e",
+                          "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=600)
+    assert out.returncode == 0, out.stderr[-2000:]
+    line = json.loads(out.stdout.strip().splitlines()[-1])
+    assert line["steps"] == 2 and line["gpu_launches"] % 2 == 0
+    assert sum(p.stat().st_size for p in tmp_path.iterdir()) <= 64 * 1000 * 1000
+    rows = np.load(tmp_path / "distances_rows.npy")
+    sample = np.load(tmp_path / "distances_sample.npy")
+    sums = np.load(tmp_path / "distances_row_sums.npy")
+    assert rows.dtype == np.float64 and sample.dtype == np.float32 and sums.dtype == np.float64
+    assert 0 < rows.size < n and sample.shape == (rows.size, n) and sums.shape == (n,)
+    D = ShardedDegreeHSD(engine.DeviceGraph.upload(powerlaw_graph(n, 5, seed=0)), hops).step()
+    torch.cuda.synchronize()
+    D = D.cpu().numpy()
+    assert np.array_equal(sample, D[rows.astype(np.int64)])
+    np.testing.assert_allclose(sums, D.astype(np.float64).sum(1), rtol=1e-12)
