@@ -19,6 +19,7 @@ HEADER_SYMBOLS = [
     "hsd_pairwise_w1_merge", "hsd_pairwise_aligned", "hsd_pairwise_worker", "hsd_cheb_spmm", "hsd_laplacian_spmv", "hsd_ring_reduce", "hsd_characteristic_function", "hsd_topk_rows",
     "hsd_fp32_peak_probe", "hsd_copy2d_to_host", "hsd_mirror_upper_to_lower_host", "hsd_exact_wavelets", "hsd_ring_dense_workspace_words", "hsd_ring_signature_degree_dense",
     "hsd_ring_cols_workspace_words", "hsd_ring_counts_dense_cols", "hsd_ring_signature_from_counts",
+    "hsd_topk_merge", "hsd_topk_merge_cols",
 ]
 
 
@@ -78,6 +79,8 @@ lib.hsd_laplacian_spmv.argtypes = [_P, _P, c_int32, _P, _P, _P]
 lib.hsd_ring_reduce.argtypes = [_P, c_int32, c_int32, c_int32, _P, _P, _P, c_int32, c_int32, _P, _P, c_int64, _P]
 lib.hsd_characteristic_function.argtypes = [_P, c_int64, c_int32, c_int32, _P, c_int32, _P, _P]
 lib.hsd_topk_rows.argtypes = [_P, c_int64, c_int32, c_int32, c_int32, c_int32, _P, _P, _P, _P]
+lib.hsd_topk_merge.argtypes = [_P, _P, c_int32, c_int64, c_int32, c_int32, c_int32, _P, _P, _P]
+lib.hsd_topk_merge_cols.argtypes = [_P, c_int64, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, _P, _P, _P]
 lib.hsd_fp32_peak_probe.argtypes = [_P, c_int32, POINTER(c_int64), _P]
 lib.hsd_exact_wavelets.argtypes = [_P, c_int64, _P, c_int32, c_double, c_double, c_int32, _P, c_int64, _P]
 lib.hsd_copy2d_to_host.argtypes = [_P, c_int64, _P, c_int64, c_int64, c_int64, _P]

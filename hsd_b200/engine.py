@@ -14,7 +14,7 @@ from typing import Optional, Tuple
 import numpy as np
 import torch
 
-from ._lib import check, lib
+from ._lib import HSDError, check, lib
 from .graph import CSRGraph
 
 PAIR_TILE = 128
@@ -407,6 +407,188 @@ def topk_rows(D: torch.Tensor, k: int, self_col0: int = 0, n_cols: Optional[int]
     val = torch.empty((n_rows, k), dtype=torch.float32, device=D.device)
     check(lib.hsd_topk_rows(D.data_ptr(), D.stride(0), n_rows, n_cols, k, self_col0, _ptr(col_mask),
                             _ptr(idx), _ptr(val), _stream()))
+    return idx, val
+
+
+def topk_merge(idx_in: torch.Tensor, val_in: torch.Tensor, idx_io: torch.Tensor, val_io: torch.Tensor,
+               idx_offset: int = 0) -> None:
+    """Merge candidate lists idx_in / val_in [n_lists, n_rows, k] (or [n_rows, k]: one list) into the
+    running lists idx_io / val_io [n_rows, k] in place (hsd_topk_merge); idx_offset is added to the
+    candidate ids that are not -1.  Every list is ordered by (distance, id) and padded with -1 / +inf."""
+    if idx_in.dim() == 2:
+        idx_in, val_in = idx_in.unsqueeze(0), val_in.unsqueeze(0)
+    n_lists, n_rows, k = idx_in.shape
+    if (val_in.shape != idx_in.shape or tuple(idx_io.shape) != (n_rows, k) or val_io.shape != idx_io.shape
+            or idx_in.dtype != torch.int32 or idx_io.dtype != torch.int32
+            or val_in.dtype != torch.float32 or val_io.dtype != torch.float32):
+        raise ValueError("idx / val must be int32 / float32 lists of matching shapes [n_lists, n_rows, k] -> [n_rows, k]")
+    check(lib.hsd_topk_merge(_ptr(idx_in), _ptr(val_in), n_lists, n_rows * k, idx_offset, n_rows, k,
+                             _ptr(idx_io), _ptr(val_io), _stream()))
+
+
+def topk_merge_cols(blk: torch.Tensor, k: int, idx_io: torch.Tensor, val_io: torch.Tensor, c_begin: int = 0,
+                    n_cols: Optional[int] = None, row_node0: int = 0, col_node0: int = 0) -> None:
+    """Column pass of a k-NN panel (hsd_topk_merge_cols): for every block column c in [c_begin, n_cols)
+    merge the candidates (blk[r, c], row_node0 + r) into the running list idx_io / val_io[col_node0 + c]."""
+    if blk.dtype != torch.float32 or blk.stride(1) != 1:
+        raise ValueError("blk must be a row-major float32 CUDA tensor")
+    n_cols = blk.shape[1] if n_cols is None else n_cols
+    if idx_io.shape[1] != k or val_io.shape != idx_io.shape or col_node0 + n_cols > idx_io.shape[0]:
+        raise ValueError("running lists must be [>= col_node0 + n_cols, k]")
+    check(lib.hsd_topk_merge_cols(blk.data_ptr(), blk.stride(0), blk.shape[0], c_begin, n_cols, row_node0,
+                                  col_node0, k, _ptr(idx_io), _ptr(val_io), _stream()))
+
+
+# --------------------------------------------------------------------------
+# k nearest neighbours by row panels: the matrix never exists as a whole
+# --------------------------------------------------------------------------
+KNN_BLOCK_FRACTION = 0.5    # default panel budget: this share of the free device memory
+KNN_PANELS_PER_RANK = 8     # world > 1: at least this many panels per rank, so that dealing balances
+
+
+def knn_panel_rows(n: int, block_bytes: int, world: int = 1) -> int:
+    """Rows R of a k-NN panel: the largest multiple of 128 whose widest panel buffer (R x roundup(N, 4)
+    floats) fits `block_bytes`, at least 128; N (one panel) when the whole matrix fits.  With several
+    ranks the panels are kept small enough that every rank gets about KNN_PANELS_PER_RANK of them."""
+    r = max(PAIR_TILE, int(block_bytes) // (4 * roundup(n, 4)) // PAIR_TILE * PAIR_TILE)
+    if world > 1:
+        r = min(r, max(PAIR_TILE, n // (KNN_PANELS_PER_RANK * world) // PAIR_TILE * PAIR_TILE))
+    return n if r >= n else r
+
+
+def knn_panels(n: int, panel_rows: int):
+    """[(r0, r1)]: the rows [0, N) in consecutive panels of `panel_rows` rows (a multiple of 128, or
+    >= N for one panel); the last panel takes the remainder."""
+    if panel_rows >= n:
+        return [(0, n)] if n else []
+    if panel_rows <= 0 or panel_rows % PAIR_TILE:
+        raise ValueError("panel_rows must be a positive multiple of 128")
+    return [(r0, min(r0 + panel_rows, n)) for r0 in range(0, n, panel_rows)]
+
+
+def knn_panel_work(n: int, r0: int, r1: int) -> float:
+    """Pairs a panel computes: its R x R / 2 diagonal square and the R x (N - r1) rectangle."""
+    R = r1 - r0
+    return R * (n - r0 - R / 2)
+
+
+def knn_deal(n: int, panels, world: int):
+    """Panels per rank, longest work first onto the least-loaded rank (ties: lower panel start, lower
+    rank), each rank's list in ascending row order.  Deterministic: every rank derives the same deal.
+    The largest load exceeds the mean by less than one panel's work."""
+    load = [0.0] * world
+    mine = [[] for _ in range(world)]
+    for p in sorted(panels, key=lambda p: (-knn_panel_work(n, *p), p[0])):
+        r = min(range(world), key=lambda i: (load[i], i))
+        load[r] += knn_panel_work(n, *p)
+        mine[r].append(p)
+    return [sorted(m) for m in mine]
+
+
+def _knn_table(dg: DeviceGraph, hops: int, empty: str, rank: int, world: int, group):
+    """(sigT, status flags OR-ed over the ranks) for the k-NN sweep.  With a process group, each rank
+    computes its dealt sources and the table is gathered (ShardedDegreeHSD); else on this device."""
+    import torch.distributed as dist
+    k_used = dg.k_used(hops)
+    if world > 1 and dist.is_available() and dist.is_initialized():
+        from .sharded import ShardedDegreeHSD, agree_status
+        plan = ShardedDegreeHSD(dg, hops, rank, world, group=group, empty=empty)
+        plan.signatures()
+        plan.gather()
+        signature_transpose(plan.sig_all, k_used, plan.sigT, 0, src_rows=plan.table_row)
+        return plan.sigT, agree_status(plan.status, world, group)
+    sig, _, _, status = ring_signature_degree(dg, hops, empty=empty)
+    sigT = alloc_signature_table(k_used, dg.n, sig.device)
+    signature_transpose(sig, k_used, sigT, 0)
+    return sigT, int(status.item())
+
+
+def degree_knn(dg: DeviceGraph, hops: int, k: int, empty: str = "raise", block_bytes: Optional[int] = None,
+               panel_rows: Optional[int] = None, rank: int = 0, world: int = 1, group=None,
+               pair_events: Optional[list] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """k nearest neighbours of every node under the degree-mode distance, without the N x N matrix:
+    (idx int32[N, k], dist float32[N, k]) ordered by (distance, node id), -1 / +inf where a node has
+    fewer than k others — bit for bit topk_rows(degree_distance_device(dg, hops)[0], k).
+
+    The rows are swept in panels P = [r0, r1).  Per panel, one buffer B[R][roundup(N - r0, 4)] receives
+    the diagonal square (one symmetric pairwise launch) and the rectangle rows P x columns [r1, N)
+    (one plain launch); hsd_topk_rows + hsd_topk_merge fold B's rows into the lists of P, and
+    hsd_topk_merge_cols folds B's columns into the lists of the nodes after P.  Every unordered pair is
+    computed once and reaches each of its two nodes' lists once.  Only B (at most `block_bytes`,
+    default KNN_BLOCK_FRACTION of the free memory) and the lists are resident; when the whole matrix
+    fits there is one panel, i.e. the launches of the resident path.
+    panel_rows: force the panel height (a multiple of 128; tests).
+    world > 1 with an initialised process group: every rank builds its dealt signatures (ShardedDegreeHSD),
+    sweeps its share of the panels (knn_deal) into its own lists, and one all-gather + hsd_topk_merge gives
+    every rank the whole result.  Without a process group the table is built on this device and this
+    rank's PARTIAL lists are returned (ranks emulated in one process; merge them with topk_merge).
+    pair_events: a list that receives (r0, r1, start, end) per panel swept here, start / end being CUDA events
+    around the panel's pairwise launches."""
+    import torch.distributed as dist
+    if empty not in ("raise", "zero"):
+        raise ValueError("empty must be 'raise' or 'zero'")
+    if not 1 <= k <= 64:      # the library's error, as hsd_topk_rows reports it on the resident matrix
+        raise HSDError(-1, "degree_knn: k must be in 1..64")
+    if not 0 <= rank < world:
+        raise ValueError("rank must be in 0..world-1")
+    n = dg.n
+    dev = dg.rowptr.device
+    k_used = dg.k_used(hops)
+    sigT, flags = _knn_table(dg, hops, empty, rank, world, group)
+    if empty == "raise" and flags & 1:
+        raise EmptyRingError("Distribution can't be empty.")
+    if panel_rows is None:
+        if block_bytes is None:    # free memory, counting blocks torch's allocator holds but does not use
+            free = torch.cuda.mem_get_info(dev)[0] + torch.cuda.memory_reserved(dev) - torch.cuda.memory_allocated(dev)
+            block_bytes = int(free * KNN_BLOCK_FRACTION)
+        panel_rows = knn_panel_rows(n, block_bytes, world)
+    mine = knn_deal(n, knn_panels(n, panel_rows), world)[rank]
+    idx = torch.full((n, k), -1, dtype=torch.int32, device=dev)
+    val = torch.full((n, k), float("inf"), dtype=torch.float32, device=dev)
+    if mine:
+        cap = max((r1 - r0) * roundup(n - r0, 4) for r0, r1 in mine)
+        try:                                                             # one panel buffer for the sweep
+            buf = torch.empty(cap, dtype=torch.float32, device=dev)
+        except torch.OutOfMemoryError:   # the budget counted cached blocks the allocator had split: release them
+            torch.cuda.empty_cache()
+            buf = torch.empty(cap, dtype=torch.float32, device=dev)
+        r_max = max(r1 - r0 for r0, r1 in mine)
+        t_idx = torch.empty((r_max, k), dtype=torch.int32, device=dev)
+        t_val = torch.empty((r_max, k), dtype=torch.float32, device=dev)
+        st = _stream()
+        for r0, r1 in mine:
+            R, ld = r1 - r0, roundup(n - r0, 4)
+            B = buf[:R * ld].view(R, ld)
+            if pair_events is not None:
+                ev = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
+                ev[0].record()
+            # block row r = node r0 + r, block column c = node r0 + c
+            check(lib.hsd_pairwise_l1(_ptr(sigT), k_used, sigT.stride(0), r0, R, r0, R, 1, B.data_ptr(), ld, st))
+            if r1 < n:   # R is a multiple of 128 here: the rectangle starts 16-byte aligned
+                check(lib.hsd_pairwise_l1(_ptr(sigT), k_used, sigT.stride(0), r0, R, r1, n - r1, 0,
+                                          B.data_ptr() + 4 * R, ld, st))
+            if pair_events is not None:
+                ev[1].record()
+                pair_events.append((r0, r1) + ev)
+            # row pass: the lists of P see columns [r0, N) here; columns before r0 arrived by earlier column passes
+            if r0 == 0:      # nothing has reached rows [0, R) yet: select straight into the lists
+                check(lib.hsd_topk_rows(B.data_ptr(), ld, R, n - r0, k, 0, None, _ptr(idx), _ptr(val), st))
+            else:
+                check(lib.hsd_topk_rows(B.data_ptr(), ld, R, n - r0, k, 0, None, _ptr(t_idx), _ptr(t_val), st))
+                check(lib.hsd_topk_merge(_ptr(t_idx), _ptr(t_val), 1, R * k, r0, R, k,
+                                         idx[r0:].data_ptr(), val[r0:].data_ptr(), st))
+            # column pass: rows of P become candidates of the nodes after P
+            if r1 < n:
+                check(lib.hsd_topk_merge_cols(B.data_ptr(), ld, R, R, n - r0, r0, r0, k, _ptr(idx), _ptr(val), st))
+        del buf, t_idx, t_val
+    if world > 1 and dist.is_available() and dist.is_initialized():
+        all_idx = torch.empty((world, n, k), dtype=torch.int32, device=dev)
+        all_val = torch.empty((world, n, k), dtype=torch.float32, device=dev)
+        dist.all_gather_into_tensor(all_idx, idx, group=group)
+        dist.all_gather_into_tensor(all_val, val, group=group)
+        idx.fill_(-1)
+        val.fill_(float("inf"))
+        topk_merge(all_idx, all_val, idx, val)
     return idx, val
 
 

@@ -245,14 +245,40 @@ class HSD(object):
         return D.cpu().numpy().astype(np.float64, copy=False)
 
     @on_model_device
-    def nearest_neighbors(self, k, scale=None, approx=False):
+    def nearest_neighbors(self, k, scale=None, approx=False, block_bytes=None):
         """(idx, dist): the k structurally closest nodes of every node, selected on the device
-        from the resident distance matrix — what a precomputed-metric KNN (tools/evaluate.py:61-69)
-        needs, without moving the N x N matrix to the host.  idx are node indices (model.nodes)."""
+        — what a precomputed-metric KNN (tools/evaluate.py:61-69) needs, without moving the N x N
+        matrix to the host.  idx are node indices (model.nodes), ordered by (distance, index).
+        Degree mode sweeps the matrix in row panels of at most ``block_bytes`` (default: half the
+        free device memory) and never holds it whole (engine.degree_knn), so graphs whose matrix
+        exceeds the device memory work too; wavelet mode selects from the resident matrix."""
+        if self.signal == "degree":
+            dg = self._device_graph(include_zero=(self.empty == "zero"))
+            idx, val = engine.degree_knn(dg, self.hop, k, empty=self.empty, block_bytes=block_bytes)
+            return idx.cpu().numpy(), val.cpu().numpy()
         D = self.structural_distance_device(scale, approx)
         if D.dtype != torch.float32:
             D = D.to(torch.float32)
         idx, val = engine.topk_rows(D.contiguous(), k)
+        return idx.cpu().numpy(), val.cpu().numpy()
+
+    @on_model_device
+    def nearest_neighbors_sharded(self, k, rank, world, group=None, block_bytes=None):
+        """nearest_neighbors over `world` GPUs (degree mode; one process per GPU, torch.distributed
+        initialised): every rank builds its dealt share of the signatures and sweeps its share of the
+        row panels; every rank returns the whole (idx, dist), equal to the one-GPU result bit for bit."""
+        if self.signal != "degree":
+            raise NotImplementedError("nearest_neighbors_sharded is degree mode only (signal='degree')")
+        if not 0 <= rank < world:
+            raise ValueError("rank must be in 0..world-1")
+        import torch.distributed as dist
+        if world > 1 and not (dist.is_available() and dist.is_initialized()):
+            # without a process group the ranks' lists could not be combined: this rank's would be partial
+            raise RuntimeError("nearest_neighbors_sharded with world > 1 needs an initialised torch.distributed "
+                               "process group (one process per GPU)")
+        dg = self._device_graph(include_zero=(self.empty == "zero"))
+        idx, val = engine.degree_knn(dg, self.hop, k, empty=self.empty, block_bytes=block_bytes,
+                                     rank=rank, world=world, group=group)
         return idx.cpu().numpy(), val.cpu().numpy()
 
     @on_model_device

@@ -68,6 +68,26 @@ def agree_status(status: torch.Tensor, world: int, group=None) -> int:
     return int(status.reshape(-1)[0].item())
 
 
+def agree_all(flag: bool, world: int, group=None, device=None) -> bool:
+    """True on every rank iff `flag` is true on every rank (a MIN all-reduce); world == 1, or no process
+    group: the local value.  Used for decisions that select which collectives the ranks issue next."""
+    if world > 1:
+        import torch.distributed as dist
+        if dist.is_available() and dist.is_initialized():
+            t = torch.tensor([1 if flag else 0], dtype=torch.int32, device=device)
+            dist.all_reduce(t, op=dist.ReduceOp.MIN, group=group)
+            return bool(t.item())
+    return bool(flag)
+
+
+def cols_workspace_words(n: int, world: int) -> int:
+    """Workspace words (hsd_ring_cols_workspace_words) of the column-split ring phase on the rank that
+    owns the most bitmap pieces: the same number on every rank."""
+    from ._lib import lib as _lib_
+    return max(int(_lib_.hsd_ring_cols_workspace_words(n, *engine.ring_cols_range(n, r, world)))
+               for r in range(world))
+
+
 def symmetric_tile_list(n: int, world: int, per: int, rank: int, tile_n: int = 128):
     """Rank `rank`'s share of the upper-triangle 128 x 128 tiles of the N x N matrix, as int32[m, 3] rows
     {first row, first column, mirror flag} of 128 x tile_n tiles (tile_n = 64 splits every tile in two).
@@ -194,7 +214,9 @@ class ShardedDegreeHSD:
             import torch.distributed as dist
             want = os.environ.get("HSD_RING_SHARD_MODE", "cols" if n >= 32768 else "rows")
             if want == "cols" and dist.is_available() and dist.is_initialized():
-                self.ring_mode = "cols"
+                # the two modes issue different collectives, so every rank must take the same one
+                if agree_all(self._cols_workspace_fits(), world, group, dev):
+                    self.ring_mode = "cols"
         self.update_mode = os.environ.get("HSD_DYN_PEER_MODE", "rows")   # see update_finish()
         self._plan_sources(dg)
         node = torch.arange(n, dtype=torch.int32, device=dev)
@@ -229,7 +251,33 @@ class ShardedDegreeHSD:
         if self.peer:
             self.out = self.out_full[:max(self.n_rows, 1), :n]
         else:
-            self.out = torch.empty((max(self.n_rows, 1), n), dtype=torch.float32, device=dev)
+            self._out = None      # allocated on first use: a plan that only builds signatures never needs it
+
+    @property
+    def out(self) -> torch.Tensor:
+        """This rank's result rows (non-peer mode: float32[n_rows, N], allocated on first use)."""
+        if self._out is None:
+            self._out = torch.empty((max(self.n_rows, 1), self.dg.n), dtype=torch.float32,
+                                    device=self.dg.rowptr.device)
+        return self._out
+
+    @out.setter
+    def out(self, value: torch.Tensor) -> None:
+        self._out = value
+
+    def _cols_workspace_fits(self) -> bool:
+        """This rank's vote for the column-split ring phase.  It keeps two N x (N / world)-bit tables per rank:
+        take it only when the largest rank's tables fit in a quarter of this device's free memory (the rule
+        engine.ring_algorithm applies to the dense variant); otherwise the row-split phase runs, with the same
+        signatures.  The ranks combine their votes with agree_all."""
+        words = cols_workspace_words(self.dg.n, self.world)
+        dev = self.dg.rowptr.device
+        ws = engine._DENSE_WS.get(("cols", dev.index if dev.index is not None else torch.cuda.current_device()))
+        have = ws.numel() * 4 if ws is not None else 0     # this rank's cached tables are reused / replaced
+        if have >= words * 4:
+            return True
+        free, _ = torch.cuda.mem_get_info(dev)
+        return words * 4 <= (free + have) // 4
 
     def _plan_sources(self, dg: engine.DeviceGraph) -> None:
         """Deal this rank's BFS sources for graph `dg` (called again by update(): the degree order,

@@ -331,6 +331,32 @@ int hsd_topk_rows(const float* D, int64_t ld, int32_t n_rows, int32_t n_cols, in
                   int32_t self_col0, const uint32_t* col_mask, int32_t* idx_out, float* val_out,
                   void* stream);
 
+/* K7 without the matrix: the k-NN lists of all N nodes are built from row panels of the distance
+ * matrix, one panel at a time (hsd_b200/engine.py::degree_knn), so only N x k results and one panel
+ * ever occupy the device.  Running lists idx_io int32[..][k] / val_io float[..][k] start as -1 / +inf;
+ * every list is sorted by (distance, node id) and padded with -1 / +inf, like hsd_topk_rows writes
+ * them.  Because that order is total, merging the top-k lists of disjoint candidate sets gives exactly
+ * the top-k of their union: the result equals hsd_topk_rows on the whole matrix bit for bit.
+ * 1 <= k <= 64, distances >= 0; no atomics, so results do not depend on the schedule.
+ *
+ * hsd_topk_merge: for rows r < n_rows, merges n_lists (1..64) candidate lists
+ *   idx_in / val_in [l * list_stride + r * k + t]   (l < n_lists; list_stride >= n_rows * k when n_lists > 1)
+ * into the running lists idx_io / val_io [r * k + t] in place; idx_offset is added to every candidate
+ * id that is not -1 (a panel's hsd_topk_rows ids are block columns).  Each candidate must be absent
+ * from the running list and from the other candidate lists (disjoint column sets).
+ *
+ * hsd_topk_merge_cols: the column pass of a panel.  blk float[n_rows][ld] (ld >= n_cols) is a block
+ * whose row r is node row_node0 + r and whose column c is node col_node0 + c; for every column
+ * c in [c_begin, n_cols) the candidates (blk[r][c], row_node0 + r), r < n_rows, are merged into the
+ * running list of node col_node0 + c, stored at idx_io / val_io [(col_node0 + c) * k + t].  The
+ * caller keeps the self pair out (c_begin past the block's diagonal). */
+int hsd_topk_merge(const int32_t* idx_in, const float* val_in, int32_t n_lists, int64_t list_stride,
+                   int32_t idx_offset, int32_t n_rows, int32_t k, int32_t* idx_io, float* val_io,
+                   void* stream);
+int hsd_topk_merge_cols(const float* blk, int64_t ld, int32_t n_rows, int32_t c_begin, int32_t n_cols,
+                        int32_t row_node0, int32_t col_node0, int32_t k, int32_t* idx_io, float* val_io,
+                        void* stream);
+
 /* ---- e2e path: ship each unordered pair once, mirror on the host --------------------
  * The reference returns the dense symmetric ndarray (model/HSD.py:100-114, dist_mat[i,j] =
  * dist_mat[j,i]).  Over PCIe the matrix is the e2e bottleneck, so the host pipeline copies only
