@@ -20,6 +20,7 @@ HEADER_SYMBOLS = [
     "hsd_fp32_peak_probe", "hsd_copy2d_to_host", "hsd_mirror_upper_to_lower_host", "hsd_exact_wavelets", "hsd_ring_dense_workspace_words", "hsd_ring_signature_degree_dense",
     "hsd_ring_cols_workspace_words", "hsd_ring_counts_dense_cols", "hsd_ring_signature_from_counts",
     "hsd_topk_merge", "hsd_topk_merge_cols",
+    "hsd_radius_count", "hsd_radius_emit_rows", "hsd_radius_emit_cols", "hsd_radius_scatter",
 ]
 
 
@@ -81,6 +82,10 @@ lib.hsd_characteristic_function.argtypes = [_P, c_int64, c_int32, c_int32, _P, c
 lib.hsd_topk_rows.argtypes = [_P, c_int64, c_int32, c_int32, c_int32, c_int32, _P, _P, _P, _P]
 lib.hsd_topk_merge.argtypes = [_P, _P, c_int32, c_int64, c_int32, c_int32, c_int32, _P, _P, _P]
 lib.hsd_topk_merge_cols.argtypes = [_P, c_int64, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, _P, _P, _P]
+lib.hsd_radius_count.argtypes = [_P, c_int32, c_int64, c_int32, c_int32, c_double, _P, c_int64, _P, _P, _P]
+lib.hsd_radius_emit_rows.argtypes = [_P, c_int32, c_int64, c_int32, c_int32, _P, c_int64, _P, c_int32, _P, _P, _P]
+lib.hsd_radius_emit_cols.argtypes = [_P, c_int32, c_int64, c_int32, c_int32, _P, c_int64, _P, c_int32, _P, _P, _P]
+lib.hsd_radius_scatter.argtypes = [_P, _P, c_int32, _P, c_int32, c_int32, _P, _P, _P, _P, _P]
 lib.hsd_fp32_peak_probe.argtypes = [_P, c_int32, POINTER(c_int64), _P]
 lib.hsd_exact_wavelets.argtypes = [_P, c_int64, _P, c_int32, c_double, c_double, c_int32, _P, c_int64, _P]
 lib.hsd_copy2d_to_host.argtypes = [_P, c_int64, _P, c_int64, c_int64, c_int64, _P]

@@ -8,6 +8,7 @@ tensors and raise otherwise.
 from __future__ import annotations
 
 import ctypes
+import math
 from dataclasses import dataclass
 from typing import Optional, Tuple
 
@@ -503,6 +504,25 @@ def _knn_table(dg: DeviceGraph, hops: int, empty: str, rank: int, world: int, gr
     return sigT, int(status.item())
 
 
+def _panel_pairwise(sigT: torch.Tensor, k_used: int, n: int, r0: int, r1: int, B: torch.Tensor, ld: int, st: int,
+                    pair_events: Optional[list] = None) -> None:
+    """Fill the panel buffer B[R][ld] of rows P = [r0, r1): block row r = node r0 + r, block column c = node
+    r0 + c.  One symmetric pairwise launch computes the diagonal square, one plain launch the rectangle
+    P x columns [r1, N); every unordered pair of the panel's upper part is computed once.
+    pair_events: receives (r0, r1, start, end), CUDA events around the two launches."""
+    R = r1 - r0
+    if pair_events is not None:
+        ev = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
+        ev[0].record()
+    check(lib.hsd_pairwise_l1(_ptr(sigT), k_used, sigT.stride(0), r0, R, r0, R, 1, B.data_ptr(), ld, st))
+    if r1 < n:   # R is a multiple of 128 here: the rectangle starts 16-byte aligned
+        check(lib.hsd_pairwise_l1(_ptr(sigT), k_used, sigT.stride(0), r0, R, r1, n - r1, 0,
+                                  B.data_ptr() + 4 * R, ld, st))
+    if pair_events is not None:
+        ev[1].record()
+        pair_events.append((r0, r1) + ev)
+
+
 def degree_knn(dg: DeviceGraph, hops: int, k: int, empty: str = "raise", block_bytes: Optional[int] = None,
                panel_rows: Optional[int] = None, rank: int = 0, world: int = 1, group=None,
                pair_events: Optional[list] = None) -> Tuple[torch.Tensor, torch.Tensor]:
@@ -559,17 +579,7 @@ def degree_knn(dg: DeviceGraph, hops: int, k: int, empty: str = "raise", block_b
         for r0, r1 in mine:
             R, ld = r1 - r0, roundup(n - r0, 4)
             B = buf[:R * ld].view(R, ld)
-            if pair_events is not None:
-                ev = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
-                ev[0].record()
-            # block row r = node r0 + r, block column c = node r0 + c
-            check(lib.hsd_pairwise_l1(_ptr(sigT), k_used, sigT.stride(0), r0, R, r0, R, 1, B.data_ptr(), ld, st))
-            if r1 < n:   # R is a multiple of 128 here: the rectangle starts 16-byte aligned
-                check(lib.hsd_pairwise_l1(_ptr(sigT), k_used, sigT.stride(0), r0, R, r1, n - r1, 0,
-                                          B.data_ptr() + 4 * R, ld, st))
-            if pair_events is not None:
-                ev[1].record()
-                pair_events.append((r0, r1) + ev)
+            _panel_pairwise(sigT, k_used, n, r0, r1, B, ld, st, pair_events)
             # row pass: the lists of P see columns [r0, N) here; columns before r0 arrived by earlier column passes
             if r0 == 0:      # nothing has reached rows [0, R) yet: select straight into the lists
                 check(lib.hsd_topk_rows(B.data_ptr(), ld, R, n - r0, k, 0, None, _ptr(idx), _ptr(val), st))
@@ -590,6 +600,233 @@ def degree_knn(dg: DeviceGraph, hops: int, k: int, empty: str = "raise", block_b
         val.fill_(float("inf"))
         topk_merge(all_idx, all_val, idx, val)
     return idx, val
+
+
+# --------------------------------------------------------------------------
+# radius graph by row panels: every pair within distance r, as a symmetric CSR
+# --------------------------------------------------------------------------
+RADIUS_PAIR_FRACTION = 0.9   # default max_pairs: this share of the memory left beside the panel buffers
+RADIUS_CHUNK_ROWS = 512      # HSD_RADIUS_CHUNK_ROWS: the column counts are kept per chunk of this many rows
+
+
+def check_radius(radius) -> float:
+    """radius as a float; ValueError when it is NaN or negative (+inf is allowed: every pair)."""
+    r = float(radius)
+    if math.isnan(r) or r < 0:
+        raise ValueError(f"radius must be >= 0 and not NaN (got {radius!r})")
+    return r
+
+
+def radius_threshold_f32(radius: float) -> np.float32:
+    """The largest float32 that does not exceed `radius` (>= 0).  For a float32 distance d,
+    d <= this value exactly when float(d) <= radius, so degree-mode panels compare in float32."""
+    r = float(radius)
+    with np.errstate(over="ignore"):
+        t = np.float32(r)                     # round to nearest: may land above r (inf above FLT_MAX)
+    if float(t) > r:
+        t = np.nextafter(t, np.float32(0))
+    return t
+
+
+def radius_panel_rows(n: int, block_bytes: int) -> int:
+    """Rows R of a radius panel: knn_panel_rows, but a row also costs its hit-bitmap row
+    (roundup(N, 4) floats + ceil(N / 32) words)."""
+    row = 4 * roundup(n, 4) + 4 * ((n + 31) // 32)
+    r = max(PAIR_TILE, int(block_bytes) // row // PAIR_TILE * PAIR_TILE)
+    return n if r >= n else r
+
+
+def radius_max_pairs(free_bytes: int, elem_bytes: int) -> int:
+    """Default cap on the stored entries (nnz): RADIUS_PAIR_FRACTION x free_bytes / (2 x (4 + elem_bytes)).
+    free_bytes is the device memory left beside the call's other buffers (radius_fixed_bytes).  An entry
+    takes 4 + elem_bytes bytes (id + distance) in the per-panel pieces and as much again in the final
+    arrays, and both coexist while the CSR is assembled (16 bytes per entry in degree mode, 24 in
+    wavelet mode)."""
+    return int(max(free_bytes, 0) * RADIUS_PAIR_FRACTION) // (2 * (4 + elem_bytes))
+
+
+def radius_fixed_bytes(n: int, panels, panel_buffer: bool = True) -> int:
+    """Device bytes a radius call holds besides its entries, for N nodes swept in `panels` [(r0, r1)]:
+    the panel buffer (float32 R_max x roundup(N, 4), degree mode only), the hit bitmap (R_max x ceil(N / 32)
+    words), the int32 row counts (R_max) and column counts (N x ceil(R_max / RADIUS_CHUNK_ROWS)), the int64
+    scan of the column counts for the current panel (as many + 1), the int64 offsets every panel's pieces keep
+    until the assembly ((R + 1) + (N - r0 + 1) per panel), and the assembly's int64 counts, indptr and cursor
+    (3 N + 1)."""
+    r_max = max((r1 - r0 for r0, r1 in panels), default=0)
+    col_counts = n * -(-r_max // RADIUS_CHUNK_ROWS)
+    b = 4 * (r_max * ((n + 31) // 32) + r_max + col_counts) + 8 * (col_counts + 1)
+    if panel_buffer:
+        b += 4 * r_max * roundup(n, 4)
+    b += 8 * sum((r1 - r0 + 1) + (n - r0 + 1) for r0, r1 in panels)
+    return b + 8 * (3 * n + 1)
+
+
+def _free_bytes(dev) -> int:
+    """Free device memory, counting blocks torch's allocator holds but does not use."""
+    return torch.cuda.mem_get_info(dev)[0] + torch.cuda.memory_reserved(dev) - torch.cuda.memory_allocated(dev)
+
+
+class _RadiusSweep:
+    """Per-panel selection (hsd_radius_count / _emit_rows / _emit_cols) and the CSR assembly
+    (hsd_radius_scatter) shared by degree_radius and radius_resident.  Pieces are kept per panel until
+    the sweep ends: (r0, row_off int64[R+1], row idx / val, col_off int64[C+1], col idx / val)."""
+
+    def __init__(self, n: int, dtype: torch.dtype, radius: float, max_pairs: int, dev):
+        self.n, self.dtype, self.dev = n, dtype, dev
+        self.elem = 4 if dtype == torch.float32 else 8
+        # float panels compare against the largest float32 <= radius (the library derives the same value)
+        self.radius = float(radius_threshold_f32(radius)) if self.elem == 4 else float(radius)
+        self.radius_asked = radius
+        self.max_pairs = int(max_pairs)
+        self.nnz = 0
+        self.pieces = []
+
+    def release(self) -> None:
+        self.pieces.clear()
+
+    def panel(self, B: torch.Tensor, ld: int, R: int, C: int, r0: int, hits: torch.Tensor,
+              row_cnt: torch.Tensor, col_cnt: torch.Tensor, st: int) -> bool:
+        """Select the hits of panel B (rows r0 + r, columns r0 + c, upper part c > r) into a row piece and
+        a column piece.  Returns False, with this sweep's pieces released, when the running nnz exceeds
+        max_pairs; that is known after the count pass, before the panel's pieces are allocated.  The
+        caller drops its own buffers and raises cap_error(): an exception raised here would keep this
+        frame, and so the panel, alive in its traceback."""
+        hits_ld = (C + 31) // 32
+        check(lib.hsd_radius_count(B.data_ptr(), self.elem, ld, R, C, self.radius, _ptr(hits), hits_ld,
+                                   _ptr(row_cnt), _ptr(col_cnt), st))
+        chunks = -(-R // RADIUS_CHUNK_ROWS)
+        row_off = torch.zeros(R + 1, dtype=torch.int64, device=self.dev)
+        col_off = torch.zeros(C * chunks + 1, dtype=torch.int64, device=self.dev)   # [c][chunk], then the total
+        torch.cumsum(row_cnt[:R], 0, out=row_off[1:])
+        torch.cumsum(col_cnt[:C * chunks], 0, out=col_off[1:])
+        total = int(row_off[-1].item())                  # the panel's one device-to-host copy
+        self.nnz += 2 * total
+        if self.nnz > self.max_pairs:
+            self.release()
+            return False
+        if total == 0:
+            return True
+        ri = torch.empty(total, dtype=torch.int32, device=self.dev)
+        rv = torch.empty(total, dtype=self.dtype, device=self.dev)
+        ci = torch.empty(total, dtype=torch.int32, device=self.dev)
+        cv = torch.empty(total, dtype=self.dtype, device=self.dev)
+        check(lib.hsd_radius_emit_rows(B.data_ptr(), self.elem, ld, R, C, _ptr(hits), hits_ld, _ptr(row_off), r0,
+                                       _ptr(ri), _ptr(rv), st))
+        check(lib.hsd_radius_emit_cols(B.data_ptr(), self.elem, ld, R, C, _ptr(hits), hits_ld, _ptr(col_off), r0,
+                                       _ptr(ci), _ptr(cv), st))
+        self.pieces.append((r0, row_off, ri, rv, col_off[::chunks].contiguous(), ci, cv))   # per column
+        return True
+
+    def cap_error(self) -> ValueError:
+        return ValueError(f"radius_neighbors: the graph at radius {self.radius_asked!r} has at least {self.nnz} "
+                          f"entries (pairs x 2), more than max_pairs = {self.max_pairs}")
+
+    def assemble(self) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+        """(indptr int64[N+1], idx int32[nnz], dist[nnz]).  Node i's row is the column pieces of every
+        panel with r0 <= i, in panel order (ids below i), then its own row piece (ids above i)."""
+        n, dev, st = self.n, self.dev, _stream()
+        counts = torch.zeros(n, dtype=torch.int64, device=dev)
+        for r0, row_off, _, _, col_off, _, _ in self.pieces:
+            counts[r0:r0 + col_off.numel() - 1] += col_off.diff()
+            counts[r0:r0 + row_off.numel() - 1] += row_off.diff()
+        indptr = torch.zeros(n + 1, dtype=torch.int64, device=dev)
+        torch.cumsum(counts, 0, out=indptr[1:])
+        del counts
+        idx = torch.empty(self.nnz, dtype=torch.int32, device=dev)
+        val = torch.empty(self.nnz, dtype=self.dtype, device=dev)
+        cursor = torch.zeros(n, dtype=torch.int64, device=dev)
+        while self.pieces:                               # each piece is freed once it is placed
+            r0, row_off, ri, rv, col_off, ci, cv = self.pieces.pop(0)
+            for off, pi, pv in ((col_off, ci, cv), (row_off, ri, rv)):
+                check(lib.hsd_radius_scatter(_ptr(pi), _ptr(pv), self.elem, _ptr(off), off.numel() - 1, r0,
+                                             _ptr(indptr), _ptr(cursor), _ptr(idx), _ptr(val), st))
+        return indptr, idx, val
+
+
+def degree_radius(dg: DeviceGraph, hops: int, radius: float, empty: str = "raise",
+                  block_bytes: Optional[int] = None, panel_rows: Optional[int] = None,
+                  max_pairs: Optional[int] = None,
+                  pair_events: Optional[list] = None) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """Radius graph of the degree-mode distance without the N x N matrix: (indptr int64[N+1], idx int32[nnz],
+    dist float32[nnz]), a CSR whose row i lists every j != i with float(D[i, j]) <= radius in ascending j,
+    D being degree_distance_device(dg, hops)[0].  Exactly symmetric, no self pairs, distance-0 pairs kept.
+
+    The rows are swept in the panels of degree_knn (same pairwise launches, same budget rule with the hit
+    bitmap counted: radius_panel_rows); per panel hsd_radius_count finds the hits of the upper part, and
+    hsd_radius_emit_rows / _emit_cols write them as the panel's rows and as the entries its columns
+    receive.  After the sweep hsd_radius_scatter assembles the CSR.  No pair is computed twice.
+    max_pairs caps nnz (default radius_max_pairs of the memory left beside radius_fixed_bytes); beyond it
+    ValueError, with the call's device buffers released.
+    pair_events: a list that receives (r0, r1, start, end) per panel, CUDA events around its pairwise launches."""
+    if empty not in ("raise", "zero"):
+        raise ValueError("empty must be 'raise' or 'zero'")
+    radius = check_radius(radius)
+    n = dg.n
+    dev = dg.rowptr.device
+    k_used = dg.k_used(hops)
+    sigT, flags = _knn_table(dg, hops, empty, 0, 1, None)
+    if empty == "raise" and flags & 1:
+        raise EmptyRingError("Distribution can't be empty.")
+    free = _free_bytes(dev)
+    if panel_rows is None:
+        panel_rows = radius_panel_rows(n, int(free * KNN_BLOCK_FRACTION) if block_bytes is None else block_bytes)
+    panels = knn_panels(n, panel_rows)
+    r_max = max((r1 - r0 for r0, r1 in panels), default=0)
+    cap = r_max * roundup(n, 4)
+    words = r_max * ((n + 31) // 32)
+    col_counts = n * -(-r_max // RADIUS_CHUNK_ROWS)
+    if max_pairs is None:
+        max_pairs = radius_max_pairs(free - radius_fixed_bytes(n, panels), 4)
+    sweep = _RadiusSweep(n, torch.float32, radius, max_pairs, dev)
+    if panels:
+        try:
+            buf = torch.empty(cap, dtype=torch.float32, device=dev)
+        except torch.OutOfMemoryError:   # the budget counted cached blocks the allocator had split: release them
+            torch.cuda.empty_cache()
+            buf = torch.empty(cap, dtype=torch.float32, device=dev)
+        hits = torch.empty(max(words, 1), dtype=torch.int32, device=dev)
+        row_cnt = torch.empty(r_max, dtype=torch.int32, device=dev)
+        col_cnt = torch.empty(col_counts, dtype=torch.int32, device=dev)
+        st = _stream()
+        for r0, r1 in panels:
+            R, C, ld = r1 - r0, n - r0, roundup(n - r0, 4)
+            B = buf[:R * ld].view(R, ld)
+            _panel_pairwise(sigT, k_used, n, r0, r1, B, ld, st, pair_events)
+            if not sweep.panel(B, ld, R, C, r0, hits, row_cnt, col_cnt, st):
+                B = buf = hits = row_cnt = col_cnt = sigT = None    # the error leaves no buffer of this call
+                raise sweep.cap_error()
+        B = buf = hits = row_cnt = col_cnt = sigT = None
+    return sweep.assemble()
+
+
+def radius_resident(D: torch.Tensor, radius: float,
+                    max_pairs: Optional[int] = None) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """Radius graph of a device-resident symmetric distance matrix D [N, N] (float32 or float64, row-major,
+    e.g. the wavelet-mode matrix): degree_radius's selection and assembly with the whole matrix as one
+    panel.  Only the upper triangle is read; the entries below it are its mirror.  Same outputs, dist in
+    D's dtype; max_pairs defaults to radius_max_pairs of the free memory beside radius_fixed_bytes."""
+    radius = check_radius(radius)
+    if D.dtype not in (torch.float32, torch.float64) or D.dim() != 2 or D.shape[0] != D.shape[1] \
+            or D.stride(1) != 1:
+        raise ValueError("D must be a square row-major float32 / float64 CUDA tensor")
+    n = D.shape[0]
+    dev = D.device
+    elem = D.element_size()
+    words = n * ((n + 31) // 32)
+    col_counts = n * -(-n // RADIUS_CHUNK_ROWS)
+    if max_pairs is None:
+        max_pairs = radius_max_pairs(_free_bytes(dev) - radius_fixed_bytes(n, [(0, n)], panel_buffer=False), elem)
+    sweep = _RadiusSweep(n, D.dtype, radius, max_pairs, dev)
+    if n:
+        hits = torch.empty(words, dtype=torch.int32, device=dev)
+        row_cnt = torch.empty(n, dtype=torch.int32, device=dev)
+        col_cnt = torch.empty(col_counts, dtype=torch.int32, device=dev)
+        ok = sweep.panel(D, D.stride(0), n, n, 0, hits, row_cnt, col_cnt, _stream())
+        hits = row_cnt = col_cnt = None
+        if not ok:
+            D = None                     # the traceback keeps this frame: it must not keep the matrix
+            raise sweep.cap_error()
+    return sweep.assemble()
 
 
 def fp32_issue_peak(iters: int = 20000, reps: int = 3) -> float:

@@ -263,6 +263,34 @@ class HSD(object):
         return idx.cpu().numpy(), val.cpu().numpy()
 
     @on_model_device
+    def radius_neighbors(self, radius, scale=None, approx=False, block_bytes=None, max_pairs=None):
+        """(indptr, indices, dist): the radius graph — every pair of nodes whose structural distance is
+        at most ``radius`` — as a canonical CSR over node indices (model.nodes): row i lists every j != i
+        with float(D[i, j]) <= radius in ascending j, D being the matrix structural_distance_device holds.
+        The graph is exactly symmetric and keeps distance-0 pairs (radius 0 lists the pairs the distance
+        cannot tell apart), so ``scipy.sparse.csr_matrix((dist, indices, indptr), shape=(N, N))`` is
+        what DBSCAN(metric="precomputed") and graph clustering take.  indptr int64[N+1], indices
+        int32[nnz], dist float32 (degree mode) / float64 (wavelet mode).
+        radius: >= 0 (+inf: every pair); NaN or negative raise ValueError.
+        block_bytes: as for nearest_neighbors — degree mode sweeps the matrix in row panels of at most
+        this size (engine.degree_radius) and never holds it whole; wavelet mode thresholds the resident
+        matrix (engine.radius_resident).
+        max_pairs: cap on nnz (stored entries, twice the pairs); the default is engine.radius_max_pairs
+        of the free device memory.  Past it ValueError, and the call's device buffers are released."""
+        radius = engine.check_radius(radius)
+        if self.signal == "degree":
+            dg = self._device_graph(include_zero=(self.empty == "zero"))
+            out = engine.degree_radius(dg, self.hop, radius, empty=self.empty, block_bytes=block_bytes,
+                                       max_pairs=max_pairs)
+        else:
+            D = self.structural_distance_device(scale, approx)
+            try:
+                out = engine.radius_resident(D, radius, max_pairs=max_pairs)
+            finally:
+                del D                    # also on the max_pairs error: its traceback keeps this frame
+        return tuple(t.cpu().numpy() for t in out)
+
+    @on_model_device
     def nearest_neighbors_sharded(self, k, rank, world, group=None, block_bytes=None):
         """nearest_neighbors over `world` GPUs (degree mode; one process per GPU, torch.distributed
         initialised): every rank builds its dealt share of the signatures and sweeps its share of the

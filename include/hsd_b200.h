@@ -357,6 +357,43 @@ int hsd_topk_merge_cols(const float* blk, int64_t ld, int32_t n_rows, int32_t c_
                         int32_t row_node0, int32_t col_node0, int32_t k, int32_t* idx_io, float* val_io,
                         void* stream);
 
+/* K7 radius graph: every pair (i, j), i != j, with D[i][j] <= radius, as a symmetric CSR graph built from
+ * the same row panels (hsd_b200/engine.py::degree_radius), so the N x N matrix never has to exist.
+ * blk is a panel of float (elem_bytes 4) or double (elem_bytes 8) values [n_rows][ld], ld >= n_cols:
+ * block row r is node r0 + r, block column c is node r0 + c, and only its upper part (c > r) is read —
+ * it holds every pair the panel owns once.  hits uint32[n_rows][hits_ld], hits_ld >= ceil(n_cols / 32),
+ * is the hit bitmap (bit c % 32 of word [r][c / 32]: blk[r][c] <= radius, c > r); radius >= 0, not NaN,
+ * +inf allowed.  The compare is (double)blk[r][c] <= radius; for float blocks it is done as
+ * blk[r][c] <= the largest float not above radius.  No atomics decide a position: results do not depend
+ * on the schedule.
+ *
+ * hsd_radius_count: writes hits (words holding a column c > r), row_cnt int32[n_rows] (hits of row r) and
+ *   col_cnt int32[n_cols][n_chunks] (hits of column c over the rows r < c of chunk q, rows
+ *   [q * HSD_RADIUS_CHUNK_ROWS, (q + 1) * HSD_RADIUS_CHUNK_ROWS), n_chunks = ceil(n_rows / HSD_RADIUS_CHUNK_ROWS));
+ *   both counts are zeroed first.
+ * hsd_radius_emit_rows: row r's hits in ascending c, (col_node0 + c, blk[r][c]), at idx_out / val_out
+ *   [row_off[r] ..], row_off int64 the exclusive scan of row_cnt.
+ * hsd_radius_emit_cols: column c's hits in ascending r, (row_node0 + r, blk[r][c]), at idx_out / val_out
+ *   [col_off[c][0] ..], col_off int64[n_cols][n_chunks] the exclusive scan of col_cnt in that (row-major) order.
+ * hsd_radius_scatter: assembly of the CSR.  Segment s < n_seg is node node0 + s's piece
+ *   idx / val [off[s], off[s + 1]) (off int64[n_seg + 1], e.g. a row_off or col_off with its total
+ *   appended); it is copied to idx_out / val_out at indptr[node] + cursor[node], and cursor[node] grows by
+ *   its length.  Called per piece in panel order, column piece before row piece, every output row comes
+ *   out ascending. */
+#define HSD_RADIUS_CHUNK_ROWS 512
+int hsd_radius_count(const void* blk, int32_t elem_bytes, int64_t ld, int32_t n_rows, int32_t n_cols,
+                     double radius, uint32_t* hits, int64_t hits_ld, int32_t* row_cnt, int32_t* col_cnt,
+                     void* stream);
+int hsd_radius_emit_rows(const void* blk, int32_t elem_bytes, int64_t ld, int32_t n_rows, int32_t n_cols,
+                         const uint32_t* hits, int64_t hits_ld, const int64_t* row_off, int32_t col_node0,
+                         int32_t* idx_out, void* val_out, void* stream);
+int hsd_radius_emit_cols(const void* blk, int32_t elem_bytes, int64_t ld, int32_t n_rows, int32_t n_cols,
+                         const uint32_t* hits, int64_t hits_ld, const int64_t* col_off, int32_t row_node0,
+                         int32_t* idx_out, void* val_out, void* stream);
+int hsd_radius_scatter(const int32_t* idx, const void* val, int32_t elem_bytes, const int64_t* off,
+                       int32_t n_seg, int32_t node0, const int64_t* indptr, int64_t* cursor,
+                       int32_t* idx_out, void* val_out, void* stream);
+
 /* ---- e2e path: ship each unordered pair once, mirror on the host --------------------
  * The reference returns the dense symmetric ndarray (model/HSD.py:100-114, dist_mat[i,j] =
  * dist_mat[j,i]).  Over PCIe the matrix is the e2e bottleneck, so the host pipeline copies only
