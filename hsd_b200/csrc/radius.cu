@@ -14,6 +14,9 @@
 //                     spans 256 consecutive columns, so a bitmap row read is one 32-byte sector) and writes
 //                     (row_node0 + r, B[r][c]) in ascending r at col_off[c][chunk]: the lower entries the
 //                     panel's columns receive.  The row chunks give a tall panel enough CTAs to hide latency;
+//   radius_merge_parts  the ranks' partial CSRs of a sharded sweep (engine.degree_radius with world > 1) into
+//                     one: each entry's slot is its rank among its row's entries of every part, from binary
+//                     searches (no atomics), so hub rows of N - 1 entries balance like short ones;
 //   radius_scatter    assembly: 8 lanes per segment (a node's piece of one panel) copy the piece to
 //                     idx_out / val_out at indptr[node] + cursor[node] and advances the cursor.  Called
 //                     once per piece in panel order, column piece before row piece, so every output row
@@ -37,6 +40,9 @@ constexpr int CE_UNROLL = 8;                       // bitmap loads in flight per
 constexpr int CHUNK = HSD_RADIUS_CHUNK_ROWS;        // rows per column-count chunk
 constexpr int RS_THREADS = 256;                    // scatter: threads per CTA
 constexpr int RS_GROUP = 8;                        // scatter: lanes per segment (~20 neighbours per node: short)
+constexpr int RM_THREADS = 256;                    // merge of the ranks' parts: threads per CTA
+constexpr int RM_MAX_PARTS = 64;                   // parts a merge takes (their starts live in shared memory)
+constexpr int RM_CTAS_PER_SM = 8;                  // merge grid: CTAs per SM of the grid-stride loop
 
 template <typename T>
 __global__ void __launch_bounds__(RC_THREADS)
@@ -168,6 +174,58 @@ radius_scatter_kernel(const int32_t* __restrict__ idx, const T* __restrict__ val
     if (g == 0) cursor[node] += len;
 }
 
+// first index t in [lo, hi) with key < a[t] (upper) or key <= a[t] (lower); hi when there is none
+template <bool UPPER, typename K>
+__device__ __forceinline__ int64_t bound_in(const K* __restrict__ a, int64_t lo, int64_t hi, K key) {
+    while (lo < hi) {
+        const int64_t mid = (lo + hi) >> 1;
+        if (UPPER ? a[mid] <= key : a[mid] < key) lo = mid + 1;
+        else hi = mid;
+    }
+    return lo;
+}
+
+// One thread per input entry (grid-stride).  Part starts in the flat entry space are a block-wide scan of the
+// parts' sizes in shared memory; entry e of part p, row i, at position k of its row goes to
+// indptr[i] + k + sum_{q<p} upper_bound(row i of q, id) + sum_{q>p} lower_bound(row i of q, id): the rank of
+// (id, p, k) among the row's entries of all parts, so the slots form a permutation whatever the schedule.
+template <typename V>
+__global__ void __launch_bounds__(RM_THREADS)
+radius_merge_parts_kernel(int n_parts, int n_rows, const int64_t* __restrict__ part_indptr,
+                          const int64_t* __restrict__ part_base, const int32_t* __restrict__ idx,
+                          const V* __restrict__ val, const int64_t* __restrict__ indptr,
+                          int32_t* __restrict__ idx_out, V* __restrict__ val_out) {
+    __shared__ int64_t start[RM_MAX_PARTS + 1];                       // start[p]: part p's first flat entry
+    const int64_t ld = (int64_t)n_rows + 1;
+    if (threadIdx.x == 0) {
+        int64_t s = 0;
+        for (int p = 0; p < n_parts; ++p) {
+            start[p] = s;
+            s += part_indptr[p * ld + n_rows] - part_indptr[p * ld];
+        }
+        start[n_parts] = s;
+    }
+    __syncthreads();
+    const int64_t total = start[n_parts];
+    for (int64_t e = (int64_t)blockIdx.x * RM_THREADS + threadIdx.x; e < total; e += (int64_t)gridDim.x * RM_THREADS) {
+        const int p = (int)bound_in<true>(start, 0, n_parts, e) - 1;   // the last part starting at or before e
+        const int64_t* ip = part_indptr + p * ld;
+        const int64_t k = ip[0] + (e - start[p]);                     // offset in part p's own indptr
+        const int i = (int)bound_in<true>(ip, 0, n_rows + 1, k) - 1;   // row of k (empty rows skipped)
+        const int32_t id = idx[part_base[p] + k];
+        int64_t slot = indptr[i] + (k - ip[i]);
+        for (int q = 0; q < n_parts; ++q) {
+            if (q == p) continue;
+            const int64_t* iq = part_indptr + q * ld;
+            const int32_t* row = idx + part_base[q];
+            const int64_t lo = iq[i], hi = iq[i + 1];
+            slot += (q < p ? bound_in<true>(row, lo, hi, id) : bound_in<false>(row, lo, hi, id)) - lo;
+        }
+        idx_out[slot] = id;
+        val_out[slot] = val[part_base[p] + k];
+    }
+}
+
 // the largest T that does not exceed radius (radius >= 0, not NaN): `D <= it` equals `(double)D <= radius`
 template <typename T>
 static T threshold_of(double radius) {
@@ -278,6 +336,33 @@ extern "C" int hsd_radius_scatter(const int32_t* idx, const void* val, int32_t e
     else
         radius_scatter_kernel<double><<<grid, RS_THREADS, 0, st>>>(idx, (const double*)val, off, n_seg, node0,
                                                                        indptr, cursor, idx_out, (double*)val_out);
+    HSD_CUDA_TRY(cudaGetLastError());
+    return HSD_OK;
+}
+
+extern "C" int hsd_radius_merge_parts(int32_t n_parts, int32_t n_rows, const int64_t* part_indptr,
+                                      const int64_t* part_base, const int32_t* idx, const void* val,
+                                      int32_t elem_bytes, const int64_t* indptr, int32_t* idx_out, void* val_out,
+                                      void* stream) {
+    using namespace hsd;
+    HSD_REQUIRE(part_indptr && part_base && idx && val && indptr && idx_out && val_out, "null pointer");
+    HSD_REQUIRE(elem_bytes == 4 || elem_bytes == 8, "elem_bytes must be 4 (float) or 8 (double)");
+    HSD_REQUIRE(n_parts >= 1 && n_parts <= RM_MAX_PARTS, "n_parts must be in 1..64");
+    HSD_REQUIRE(n_rows >= 0, "bad sizes (n_rows must be >= 0)");
+    if (n_rows == 0) return HSD_OK;
+    int dev = 0, sms = 0;
+    HSD_CUDA_TRY(cudaGetDevice(&dev));
+    HSD_CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    const unsigned grid = (unsigned)(sms * RM_CTAS_PER_SM);
+    const cudaStream_t st = (cudaStream_t)stream;
+    if (elem_bytes == 4)     // the distances are copied as bit patterns
+        radius_merge_parts_kernel<uint32_t><<<grid, RM_THREADS, 0, st>>>(n_parts, n_rows, part_indptr, part_base, idx,
+                                                                         (const uint32_t*)val, indptr, idx_out,
+                                                                         (uint32_t*)val_out);
+    else
+        radius_merge_parts_kernel<uint64_t><<<grid, RM_THREADS, 0, st>>>(n_parts, n_rows, part_indptr, part_base, idx,
+                                                                         (const uint64_t*)val, indptr, idx_out,
+                                                                         (uint64_t*)val_out);
     HSD_CUDA_TRY(cudaGetLastError());
     return HSD_OK;
 }

@@ -628,11 +628,14 @@ def radius_threshold_f32(radius: float) -> np.float32:
     return t
 
 
-def radius_panel_rows(n: int, block_bytes: int) -> int:
+def radius_panel_rows(n: int, block_bytes: int, world: int = 1) -> int:
     """Rows R of a radius panel: knn_panel_rows, but a row also costs its hit-bitmap row
-    (roundup(N, 4) floats + ceil(N / 32) words)."""
+    (roundup(N, 4) floats + ceil(N / 32) words).  With several ranks the panels are capped like
+    knn_panel_rows caps them, so that every rank gets about KNN_PANELS_PER_RANK of them."""
     row = 4 * roundup(n, 4) + 4 * ((n + 31) // 32)
     r = max(PAIR_TILE, int(block_bytes) // row // PAIR_TILE * PAIR_TILE)
+    if world > 1:
+        r = min(r, max(PAIR_TILE, n // (KNN_PANELS_PER_RANK * world) // PAIR_TILE * PAIR_TILE))
     return n if r >= n else r
 
 
@@ -643,6 +646,21 @@ def radius_max_pairs(free_bytes: int, elem_bytes: int) -> int:
     arrays, and both coexist while the CSR is assembled (16 bytes per entry in degree mode, 24 in
     wavelet mode)."""
     return int(max(free_bytes, 0) * RADIUS_PAIR_FRACTION) // (2 * (4 + elem_bytes))
+
+
+def radius_sharded_max_pairs(free_bytes: int) -> int:
+    """Default cap on the global nnz of a radius graph swept by several ranks (degree mode):
+    RADIUS_PAIR_FRACTION x free_bytes / 24.  Every rank ends up holding each global entry twice, as the
+    gathered parts and as the merged CSR (id + float32 distance: 8 + 8 bytes), next to its own partial
+    CSR (8 bytes per entry, at most the global count).  free_bytes is the device memory left beside
+    radius_fixed_bytes of the rank's panels and the gathered indptrs."""
+    return int(max(free_bytes, 0) * RADIUS_PAIR_FRACTION) // 24
+
+
+def radius_cap_error(radius, nnz: int, max_pairs: int) -> ValueError:
+    """The error of a radius graph past its cap (nnz counts stored entries: pairs x 2)."""
+    return ValueError(f"radius_neighbors: the graph at radius {radius!r} has at least {nnz} "
+                      f"entries (pairs x 2), more than max_pairs = {max_pairs}")
 
 
 def radius_fixed_bytes(n: int, panels, panel_buffer: bool = True) -> int:
@@ -718,8 +736,7 @@ class _RadiusSweep:
         return True
 
     def cap_error(self) -> ValueError:
-        return ValueError(f"radius_neighbors: the graph at radius {self.radius_asked!r} has at least {self.nnz} "
-                          f"entries (pairs x 2), more than max_pairs = {self.max_pairs}")
+        return radius_cap_error(self.radius_asked, self.nnz, self.max_pairs)
 
     def assemble(self) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
         """(indptr int64[N+1], idx int32[nnz], dist[nnz]).  Node i's row is the column pieces of every
@@ -745,7 +762,7 @@ class _RadiusSweep:
 
 def degree_radius(dg: DeviceGraph, hops: int, radius: float, empty: str = "raise",
                   block_bytes: Optional[int] = None, panel_rows: Optional[int] = None,
-                  max_pairs: Optional[int] = None,
+                  max_pairs: Optional[int] = None, rank: int = 0, world: int = 1, group=None,
                   pair_events: Optional[list] = None) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
     """Radius graph of the degree-mode distance without the N x N matrix: (indptr int64[N+1], idx int32[nnz],
     dist float32[nnz]), a CSR whose row i lists every j != i with float(D[i, j]) <= radius in ascending j,
@@ -757,28 +774,51 @@ def degree_radius(dg: DeviceGraph, hops: int, radius: float, empty: str = "raise
     receive.  After the sweep hsd_radius_scatter assembles the CSR.  No pair is computed twice.
     max_pairs caps nnz (default radius_max_pairs of the memory left beside radius_fixed_bytes); beyond it
     ValueError, with the call's device buffers released.
+    world > 1: this rank sweeps its share of the panels (knn_deal; panels capped at about
+    N / (KNN_PANELS_PER_RANK x world) rows) into a partial CSR over all N rows.  With an initialised process
+    group every rank builds its dealt signatures (ShardedDegreeHSD), the ranks agree on the panel height and
+    on max_pairs (MIN over the group; the default is radius_sharded_max_pairs), gather every partial
+    (sharded.gather_csr_parts) and merge them with hsd_radius_merge_parts: every rank returns the whole CSR,
+    bit for bit the one-GPU result.  The cap is checked on the global nnz after the sweep, on every rank
+    together, so all ranks raise the same ValueError or none does.  Without a process group this rank's
+    PARTIAL CSR is returned (ranks emulated in one process; combine them with radius_merge).
     pair_events: a list that receives (r0, r1, start, end) per panel, CUDA events around its pairwise launches."""
+    import torch.distributed as dist
     if empty not in ("raise", "zero"):
         raise ValueError("empty must be 'raise' or 'zero'")
+    if not 0 <= rank < world:
+        raise ValueError("rank must be in 0..world-1")
     radius = check_radius(radius)
     n = dg.n
     dev = dg.rowptr.device
     k_used = dg.k_used(hops)
-    sigT, flags = _knn_table(dg, hops, empty, 0, 1, None)
+    grouped = world > 1 and dist.is_available() and dist.is_initialized()
+    sigT, flags = _knn_table(dg, hops, empty, rank, world, group)
     if empty == "raise" and flags & 1:
         raise EmptyRingError("Distribution can't be empty.")
     free = _free_bytes(dev)
     if panel_rows is None:
-        panel_rows = radius_panel_rows(n, int(free * KNN_BLOCK_FRACTION) if block_bytes is None else block_bytes)
+        panel_rows = radius_panel_rows(n, int(free * KNN_BLOCK_FRACTION) if block_bytes is None else block_bytes,
+                                       world)
+    if grouped:      # a plan taken from each rank's own free memory could differ: panels missed or swept twice
+        from .sharded import agree_min
+        panel_rows, = agree_min([panel_rows], group, dev)
     panels = knn_panels(n, panel_rows)
-    r_max = max((r1 - r0 for r0, r1 in panels), default=0)
+    mine = knn_deal(n, panels, world)[rank] if world > 1 else panels
+    r_max = max((r1 - r0 for r0, r1 in mine), default=0)
     cap = r_max * roundup(n, 4)
     words = r_max * ((n + 31) // 32)
     col_counts = n * -(-r_max // RADIUS_CHUNK_ROWS)
     if max_pairs is None:
-        max_pairs = radius_max_pairs(free - radius_fixed_bytes(n, panels), 4)
+        if world > 1:
+            max_pairs = radius_sharded_max_pairs(free - radius_fixed_bytes(n, mine) - 8 * world * (n + 1))
+        else:
+            max_pairs = radius_max_pairs(free - radius_fixed_bytes(n, panels), 4)
+    if grouped:
+        max_pairs, = agree_min([max_pairs], group, dev)
     sweep = _RadiusSweep(n, torch.float32, radius, max_pairs, dev)
-    if panels:
+    stopped = False
+    if mine:
         try:
             buf = torch.empty(cap, dtype=torch.float32, device=dev)
         except torch.OutOfMemoryError:   # the budget counted cached blocks the allocator had split: release them
@@ -788,15 +828,64 @@ def degree_radius(dg: DeviceGraph, hops: int, radius: float, empty: str = "raise
         row_cnt = torch.empty(r_max, dtype=torch.int32, device=dev)
         col_cnt = torch.empty(col_counts, dtype=torch.int32, device=dev)
         st = _stream()
-        for r0, r1 in panels:
+        for r0, r1 in mine:
             R, C, ld = r1 - r0, n - r0, roundup(n - r0, 4)
             B = buf[:R * ld].view(R, ld)
             _panel_pairwise(sigT, k_used, n, r0, r1, B, ld, st, pair_events)
             if not sweep.panel(B, ld, R, C, r0, hits, row_cnt, col_cnt, st):
-                B = buf = hits = row_cnt = col_cnt = sigT = None    # the error leaves no buffer of this call
-                raise sweep.cap_error()
-        B = buf = hits = row_cnt = col_cnt = sigT = None
-    return sweep.assemble()
+                stopped = True
+                break
+        B = buf = hits = row_cnt = col_cnt = None
+    sigT = None
+    if stopped and not grouped:          # the error leaves no buffer of this call
+        raise sweep.cap_error()
+    if not grouped:
+        return sweep.assemble()
+    from .sharded import agree_radius_cap, gather_csr_parts
+    try:                                 # every rank joins, also one that stopped: all raise together or none
+        agree_radius_cap(sweep.nnz, stopped, max_pairs, sweep.radius_asked, group, dev)
+    except ValueError:
+        sweep.release()
+        raise
+    part = sweep.assemble()
+    parts = gather_csr_parts(*part, world, group)
+    part = None
+    return _radius_merge_gathered(*parts)
+
+
+def _radius_merge_gathered(part_indptr: torch.Tensor, part_base: torch.Tensor, idx: torch.Tensor,
+                           val: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """hsd_radius_merge_parts over parts held in one pair of arrays: part p's offsets are part_indptr[p]
+    (int64[P, N+1]), its entries start at part_base[p] (int64[P]) in idx / val."""
+    n_parts, n1 = part_indptr.shape
+    indptr = torch.zeros(n1, dtype=torch.int64, device=idx.device)
+    torch.cumsum(part_indptr.diff(dim=1).sum(0), 0, out=indptr[1:])
+    nnz = int(indptr[-1].item())
+    out_idx = torch.empty(nnz, dtype=torch.int32, device=idx.device)
+    out_val = torch.empty(nnz, dtype=val.dtype, device=idx.device)
+    if nnz:
+        check(lib.hsd_radius_merge_parts(n_parts, n1 - 1, _ptr(part_indptr), _ptr(part_base), _ptr(idx), _ptr(val),
+                                         val.element_size(), _ptr(indptr), _ptr(out_idx), _ptr(out_val), _stream()))
+    return indptr, out_idx, out_val
+
+
+def radius_merge(parts) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """The CSR of the union of partial CSRs [(indptr int64[N+1], idx int32, dist)] on the device — e.g. the
+    ranks' degree_radius(..., rank=r, world=W) without a process group — by hsd_radius_merge_parts: row i
+    is the merge by id of row i of every part (1..64 parts, each row ascending, ids of a row disjoint
+    across parts)."""
+    parts = list(parts)
+    if not 1 <= len(parts) <= 64:
+        raise ValueError("radius_merge takes 1..64 parts")
+    n1 = parts[0][0].numel()
+    if any(p[0].numel() != n1 or p[0].dtype != torch.int64 or p[1].dtype != torch.int32
+           or p[2].dtype != parts[0][2].dtype or p[1].numel() != p[2].numel() for p in parts):
+        raise ValueError("parts must be (indptr int64[N+1], idx int32[nnz], dist[nnz]) of one N and one dtype")
+    sizes = [int(p[1].numel()) for p in parts]
+    dev = parts[0][0].device
+    base = torch.tensor([0] + sizes[:-1], dtype=torch.int64).cumsum(0).to(dev)
+    return _radius_merge_gathered(torch.stack([p[0] for p in parts]), base, torch.cat([p[1] for p in parts]),
+                                  torch.cat([p[2] for p in parts]))
 
 
 def radius_resident(D: torch.Tensor, radius: float,

@@ -310,6 +310,29 @@ class HSD(object):
         return idx.cpu().numpy(), val.cpu().numpy()
 
     @on_model_device
+    def radius_neighbors_sharded(self, radius, rank, world, group=None, block_bytes=None, max_pairs=None):
+        """radius_neighbors over `world` GPUs (degree mode; one process per GPU, torch.distributed
+        initialised): every rank builds its dealt share of the signatures and sweeps its share of the row
+        panels, then the ranks' partial graphs are gathered and merged on every rank.  Every rank returns
+        the whole (indptr, indices, dist), equal to the one-GPU result bit for bit.  max_pairs caps the
+        global nnz (default engine.radius_sharded_max_pairs, the MIN over the ranks); past it every rank
+        raises the same ValueError."""
+        if self.signal != "degree":
+            raise NotImplementedError("radius_neighbors_sharded is degree mode only (signal='degree')")
+        if not 0 <= rank < world:
+            raise ValueError("rank must be in 0..world-1")
+        radius = engine.check_radius(radius)
+        import torch.distributed as dist
+        if world > 1 and not (dist.is_available() and dist.is_initialized()):
+            # without a process group the ranks' graphs could not be combined: this rank's would be partial
+            raise RuntimeError("radius_neighbors_sharded with world > 1 needs an initialised torch.distributed "
+                               "process group (one process per GPU)")
+        dg = self._device_graph(include_zero=(self.empty == "zero"))
+        out = engine.degree_radius(dg, self.hop, radius, empty=self.empty, block_bytes=block_bytes,
+                                   max_pairs=max_pairs, rank=rank, world=world, group=group)
+        return tuple(t.cpu().numpy() for t in out)
+
+    @on_model_device
     def parallel_calculate_HSD(self, n_workers=3, row_signal="reference"):
         """model/HSD.py:118-137 with the worker of :140-161: hops 0..hop-1 of the zero-padded
         'aligned' distance (tools/metrics.py:151-192).  row_signal="reference" reproduces the

@@ -80,6 +80,57 @@ def agree_all(flag: bool, world: int, group=None, device=None) -> bool:
     return bool(flag)
 
 
+def agree_min(values, group=None, device=None):
+    """Element-wise MIN over the ranks of a list of integers (one int64 all-reduce): the value every rank
+    uses for a decision that must not differ between ranks, such as a plan derived from free memory."""
+    import torch.distributed as dist
+    t = torch.tensor([int(v) for v in values], dtype=torch.int64, device=device)
+    dist.all_reduce(t, op=dist.ReduceOp.MIN, group=group)
+    return [int(v) for v in t.tolist()]
+
+
+def agree_radius_cap(nnz: int, stopped: bool, max_pairs: int, radius, group=None, device=None) -> int:
+    """Global nnz of a radius graph swept by several ranks: one SUM all-reduce of (this rank's nnz, whether it
+    stopped at the cap).  Raises the same ValueError (engine.radius_cap_error) on every rank when the sum
+    exceeds max_pairs or any rank stopped; a rank past the cap must still join, or the others would hang."""
+    import torch.distributed as dist
+    t = torch.tensor([int(nnz), 1 if stopped else 0], dtype=torch.int64, device=device)
+    dist.all_reduce(t, op=dist.ReduceOp.SUM, group=group)
+    total, n_stopped = t.tolist()
+    if n_stopped or total > max_pairs:
+        raise engine.radius_cap_error(radius, total, max_pairs)
+    return total
+
+
+def gather_csr_parts(indptr: torch.Tensor, idx: torch.Tensor, val: torch.Tensor, world: int, group=None):
+    """Every rank's CSR (indptr int64[N+1] from 0, idx[nnz_r], val[nnz_r]) on every rank, without padding:
+    one all_gather_into_tensor of the indptrs gives each rank's entry count, then each rank's entries are
+    broadcast into its exact slice of one buffer per array (ranks with no entries are skipped by all ranks
+    alike).  Returns (part_indptr int64[world, N+1], part_base int64[world]: where rank r's entries start,
+    idx_all, val_all), on the inputs' device (any device the group's backend serves)."""
+    import torch.distributed as dist
+    me = dist.get_rank(group)
+    part_indptr = torch.empty(world * indptr.numel(), dtype=torch.int64, device=indptr.device)
+    dist.all_gather_into_tensor(part_indptr, indptr.contiguous(), group=group)
+    part_indptr = part_indptr.view(world, indptr.numel())
+    sizes = part_indptr[:, -1].tolist()
+    starts = [0]
+    for c in sizes:
+        starts.append(starts[-1] + c)
+    idx_all = torch.empty(starts[-1], dtype=idx.dtype, device=idx.device)
+    val_all = torch.empty(starts[-1], dtype=val.dtype, device=val.device)
+    for r in range(world):
+        if not sizes[r]:
+            continue
+        for mine, out in ((idx, idx_all), (val, val_all)):
+            piece = out[starts[r]:starts[r + 1]]
+            if r == me:
+                piece.copy_(mine)
+            dist.broadcast(piece, group=group, group_src=r)
+    part_base = torch.tensor(starts[:-1], dtype=torch.int64).to(indptr.device)
+    return part_indptr, part_base, idx_all, val_all
+
+
 def cols_workspace_words(n: int, world: int) -> int:
     """Workspace words (hsd_ring_cols_workspace_words) of the column-split ring phase on the rank that
     owns the most bitmap pieces: the same number on every rank."""

@@ -379,7 +379,15 @@ int hsd_topk_merge_cols(const float* blk, int64_t ld, int32_t n_rows, int32_t c_
  *   idx / val [off[s], off[s + 1]) (off int64[n_seg + 1], e.g. a row_off or col_off with its total
  *   appended); it is copied to idx_out / val_out at indptr[node] + cursor[node], and cursor[node] grows by
  *   its length.  Called per piece in panel order, column piece before row piece, every output row comes
- *   out ascending. */
+ *   out ascending.
+ * hsd_radius_merge_parts: the partial CSRs of a sweep split over ranks (each rank's panels give every row
+ *   some of its entries) merged into one CSR.  Part p < n_parts (1..64) has its own offsets
+ *   part_indptr[p * (n_rows + 1) + i] and its entries at idx / val [part_base[p] + part_indptr[p][i] ..
+ *   part_base[p] + part_indptr[p][i + 1]), ascending by id within a row.  indptr int64[n_rows + 1] is the
+ *   caller's scan of the summed row lengths.  Row i of idx_out / val_out [indptr[i] .. indptr[i + 1]) is the
+ *   stable merge by id of row i of every part; equal ids (absent when the parts are disjoint) are ordered by
+ *   part index, so the result never depends on the schedule.  Nothing outside [indptr[0], indptr[n_rows])
+ *   is written; the values (elem_bytes 4 or 8) are copied bit for bit. */
 #define HSD_RADIUS_CHUNK_ROWS 512
 int hsd_radius_count(const void* blk, int32_t elem_bytes, int64_t ld, int32_t n_rows, int32_t n_cols,
                      double radius, uint32_t* hits, int64_t hits_ld, int32_t* row_cnt, int32_t* col_cnt,
@@ -393,6 +401,9 @@ int hsd_radius_emit_cols(const void* blk, int32_t elem_bytes, int64_t ld, int32_
 int hsd_radius_scatter(const int32_t* idx, const void* val, int32_t elem_bytes, const int64_t* off,
                        int32_t n_seg, int32_t node0, const int64_t* indptr, int64_t* cursor,
                        int32_t* idx_out, void* val_out, void* stream);
+int hsd_radius_merge_parts(int32_t n_parts, int32_t n_rows, const int64_t* part_indptr, const int64_t* part_base,
+                           const int32_t* idx, const void* val, int32_t elem_bytes, const int64_t* indptr,
+                           int32_t* idx_out, void* val_out, void* stream);
 
 /* ---- e2e path: ship each unordered pair once, mirror on the host --------------------
  * The reference returns the dense symmetric ndarray (model/HSD.py:100-114, dist_mat[i,j] =
