@@ -22,6 +22,7 @@ HEADER_SYMBOLS = [
     "hsd_topk_merge", "hsd_topk_merge_cols",
     "hsd_radius_count", "hsd_radius_emit_rows", "hsd_radius_emit_cols", "hsd_radius_scatter",
     "hsd_radius_merge_parts",
+    "hsd_mst_panel_min", "hsd_mst_list_candidates", "hsd_single_linkage_host",
 ]
 
 
@@ -88,6 +89,9 @@ lib.hsd_radius_emit_rows.argtypes = [_P, c_int32, c_int64, c_int32, c_int32, _P,
 lib.hsd_radius_emit_cols.argtypes = [_P, c_int32, c_int64, c_int32, c_int32, _P, c_int64, _P, c_int32, _P, _P, _P]
 lib.hsd_radius_scatter.argtypes = [_P, _P, c_int32, _P, c_int32, c_int32, _P, _P, _P, _P, _P]
 lib.hsd_radius_merge_parts.argtypes = [c_int32, c_int32, _P, _P, _P, _P, c_int32, _P, _P, _P, _P]
+lib.hsd_mst_panel_min.argtypes = [_P, c_int64, c_int32, c_int32, c_int32, _P, _P, _P]
+lib.hsd_mst_list_candidates.argtypes = [_P, _P, c_int32, c_int32, _P, _P, _P, _P]
+lib.hsd_single_linkage_host.argtypes = [_P, _P, _P, c_int32, _P]
 lib.hsd_fp32_peak_probe.argtypes = [_P, c_int32, POINTER(c_int64), _P]
 lib.hsd_exact_wavelets.argtypes = [_P, c_int64, _P, c_int32, c_double, c_double, c_int32, _P, c_int64, _P]
 lib.hsd_copy2d_to_host.argtypes = [_P, c_int64, _P, c_int64, c_int64, c_int64, _P]

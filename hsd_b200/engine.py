@@ -544,19 +544,27 @@ def degree_knn(dg: DeviceGraph, hops: int, k: int, empty: str = "raise", block_b
     rank's PARTIAL lists are returned (ranks emulated in one process; merge them with topk_merge).
     pair_events: a list that receives (r0, r1, start, end) per panel swept here, start / end being CUDA events
     around the panel's pairwise launches."""
-    import torch.distributed as dist
     if empty not in ("raise", "zero"):
         raise ValueError("empty must be 'raise' or 'zero'")
     if not 1 <= k <= 64:      # the library's error, as hsd_topk_rows reports it on the resident matrix
         raise HSDError(-1, "degree_knn: k must be in 1..64")
     if not 0 <= rank < world:
         raise ValueError("rank must be in 0..world-1")
-    n = dg.n
-    dev = dg.rowptr.device
-    k_used = dg.k_used(hops)
     sigT, flags = _knn_table(dg, hops, empty, rank, world, group)
     if empty == "raise" and flags & 1:
         raise EmptyRingError("Distribution can't be empty.")
+    return _knn_sweep(sigT, dg, hops, k, block_bytes, panel_rows, rank, world, group, pair_events)
+
+
+def _knn_sweep(sigT: torch.Tensor, dg: DeviceGraph, hops: int, k: int, block_bytes: Optional[int],
+               panel_rows: Optional[int], rank: int = 0, world: int = 1, group=None,
+               pair_events: Optional[list] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """degree_knn's panel sweep and gather over a signature table it was given (_knn_table's), so that a caller
+    which sweeps the same table again (degree_mst) builds it once.  Arguments as degree_knn's, checked there."""
+    import torch.distributed as dist
+    n = dg.n
+    dev = dg.rowptr.device
+    k_used = dg.k_used(hops)
     if panel_rows is None:
         if block_bytes is None:    # free memory, counting blocks torch's allocator holds but does not use
             free = torch.cuda.mem_get_info(dev)[0] + torch.cuda.memory_reserved(dev) - torch.cuda.memory_allocated(dev)
@@ -916,6 +924,166 @@ def radius_resident(D: torch.Tensor, radius: float,
             D = None                     # the traceback keeps this frame: it must not keep the matrix
             raise sweep.cap_error()
     return sweep.assemble()
+
+
+# --------------------------------------------------------------------------
+# minimum spanning tree / single linkage by Borůvka rounds over the k-NN panels
+# --------------------------------------------------------------------------
+# k of the candidate lists that certify rounds without a sweep: the largest the top-k kernels take was the fastest
+# at 20k nodes / 3 hops and 100k nodes / 4 hops (scripts/time_mst.py, profiles/r6_mst_notes.md)
+MST_CAND_K = 64
+MST_KEY_NONE = 2 ** 63 - 1
+
+
+def _mst_contract(comp: torch.Tensor, keys: torch.Tensor, bound: Optional[torch.Tensor]):
+    """One Borůvka contraction from exact per-node keys K(d, j) (INT64 max: none).  Each component takes its
+    minimum edge under E = (dist, lo, hi): a minimum on (dist, lo), then on hi among the matches; components
+    are labelled by their smallest node, so arrays indexed by label have N entries.
+    bound: per-node bounds of list-derived keys, or None (keys from a sweep, exact).  Returns None when a
+    component's edge is not certified (its dist is not strictly below its exhausted members' smallest bound),
+    else (new comp, edges (lo, hi, dist bits) recorded once each)."""
+    n, dev = comp.numel(), comp.device
+    node = torch.arange(n, dtype=torch.int64, device=dev)
+    lab = comp.long()
+    has = keys != MST_KEY_NONE
+    j = keys & 0xFFFFFFFF
+    lo, hi = torch.minimum(node, j), torch.maximum(node, j)
+    none = torch.full((n,), MST_KEY_NONE, dtype=torch.int64, device=dev)
+    k1 = torch.where(has, (keys >> 32) << 32 | lo, none)
+    c1 = none.scatter_reduce(0, lab, k1, "amin")
+    c2 = none.scatter_reduce(0, lab, torch.where(has & (k1 == c1[lab]), hi, none), "amin")
+    roots = torch.nonzero(lab == node).squeeze(1)                          # one label per component
+    e_key, e_hi = c1[roots], c2[roots]
+    if bound is not None:
+        cb = torch.full((n,), math.inf, dtype=torch.float32, device=dev).scatter_reduce(0, lab, bound, "amin")
+        d = (e_key >> 32).int().view(torch.float32)                       # INT64 max -> NaN bits: not certified
+        if not bool((d < cb[roots]).all()):
+            return None
+    e_lo = e_key & 0xFFFFFFFF
+    other = torch.where(lab[e_lo] == roots, lab[e_hi], lab[e_lo])         # the component the edge reaches
+    parent = node.clone()
+    parent[roots] = other
+    mutual = parent[other] == roots                                        # both chose the same edge
+    keep = ~mutual | (roots < other)                                       # record it once
+    parent[roots[mutual & (roots < other)]] = roots[mutual & (roots < other)]
+    for _ in range(max(1, math.ceil(math.log2(max(roots.numel(), 2))))):   # pointer jumping to the roots
+        parent = parent[parent]
+    top = parent[lab]
+    new_lab = torch.full((n,), n, dtype=torch.int64, device=dev).scatter_reduce(0, top, node, "amin")
+    edges = (e_lo[keep], e_hi[keep], (e_key[keep] >> 32).int())
+    return new_lab[top].int(), edges
+
+
+def degree_mst(dg: DeviceGraph, hops: int, empty: str = "raise", block_bytes: Optional[int] = None,
+               cand_k: int = MST_CAND_K, panel_rows: Optional[int] = None,
+               stats: Optional[dict] = None) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """The minimum spanning tree of the complete graph under the degree-mode distance, without the N x N
+    matrix: (u int32[N-1], v int32[N-1], dist float32[N-1]), u < v, sorted by (dist, u, v) — the unique MST
+    under E(u, v) = (float(D[u, v]), u, v), i.e. Kruskal in that order on degree_distance_device(dg, hops)[0],
+    bit for bit.
+
+    Borůvka rounds: comp labels every component by its smallest node; each round every node finds its best
+    edge leaving its component, each component takes the minimum of its members' (_mst_contract), and the
+    chosen edges merge the components (at least halving their number).  A node's best edge is the minimum of
+    K(d, j) = float_bits(d) << 32 | j.  degree_knn's sweep (k = cand_k) runs once first; its lists are ordered
+    by the same (d, j), so the first entry outside the component is exact (hsd_mst_list_candidates); the lists
+    and every sweep read one signature table.  A round whose every component is certified by the lists costs
+    O(N cand_k); otherwise it is a sweep: every panel of the k-NN plan goes through the pairwise launches and
+    hsd_mst_panel_min, and every key is exact.  Every round tries the lists first, also after a sweep: a later
+    round can be certified again (profiles/r6_mst_notes.md), and a failed try costs about 1 ms at 100k nodes.
+    cand_k: 0 sweeps every round (tests); panel_rows: force the panel height (tests).  stats: a dict that
+    receives rounds, sweeps, the wall time in ms before round 1 (setup_ms: signatures and the lists; the device
+    is synchronised there), per-round wall times (round_ms; a sweep round's includes its failed list try) and
+    which rounds swept (swept)."""
+    import time
+    if empty not in ("raise", "zero"):
+        raise ValueError("empty must be 'raise' or 'zero'")
+    if not 0 <= cand_k <= 64:
+        raise ValueError("cand_k must be in 0..64")
+    n = dg.n
+    dev = dg.rowptr.device
+    k_used = dg.k_used(hops)
+    empty_out = (torch.zeros(0, dtype=torch.int32, device=dev), torch.zeros(0, dtype=torch.int32, device=dev),
+                 torch.zeros(0, dtype=torch.float32, device=dev))
+    t_call = time.perf_counter()
+    if stats is not None:
+        stats.update(rounds=0, sweeps=0, round_ms=[], swept=[], setup_ms=0.0)
+    if n == 0:
+        return empty_out
+    sigT, flags = _knn_table(dg, hops, empty, 0, 1, None)     # built once: the lists and every sweep read it
+    if empty == "raise" and flags & 1:
+        raise EmptyRingError("Distribution can't be empty.")
+    if n < 2:
+        return empty_out
+    if cand_k:
+        idx, val = _knn_sweep(sigT, dg, hops, cand_k, block_bytes, panel_rows)
+    if stats is not None:                                # the lists' sweep is not part of round 1
+        torch.cuda.synchronize(dev)
+        stats["setup_ms"] = (time.perf_counter() - t_call) * 1e3
+    st = _stream()
+    comp = torch.arange(n, dtype=torch.int32, device=dev)
+    keys = torch.empty(n, dtype=torch.int64, device=dev)
+    bound = torch.empty(n, dtype=torch.float32, device=dev)
+    parts, n_comp, buf, panels = [], n, None, None
+    while n_comp > 1:
+        t0 = time.perf_counter()
+        out = None
+        if cand_k:
+            check(lib.hsd_mst_list_candidates(_ptr(idx), _ptr(val), n, cand_k, _ptr(comp), _ptr(keys), _ptr(bound),
+                                              st))
+            out = _mst_contract(comp, keys, bound)
+        swept = out is None
+        if swept:
+            if panels is None:
+                if panel_rows is None:
+                    panel_rows = knn_panel_rows(n, int(_free_bytes(dev) * KNN_BLOCK_FRACTION)
+                                                if block_bytes is None else block_bytes)
+                panels = knn_panels(n, panel_rows)
+                cap = max((r1 - r0) * roundup(n - r0, 4) for r0, r1 in panels)
+                try:
+                    buf = torch.empty(cap, dtype=torch.float32, device=dev)
+                except torch.OutOfMemoryError:   # the budget counted cached blocks the allocator had split
+                    torch.cuda.empty_cache()
+                    buf = torch.empty(cap, dtype=torch.float32, device=dev)
+            keys.fill_(MST_KEY_NONE)
+            for r0, r1 in panels:
+                R, ld = r1 - r0, roundup(n - r0, 4)
+                B = buf[:R * ld].view(R, ld)
+                _panel_pairwise(sigT, k_used, n, r0, r1, B, ld, st)
+                check(lib.hsd_mst_panel_min(B.data_ptr(), ld, R, n - r0, r0, _ptr(comp), _ptr(keys), st))
+            out = _mst_contract(comp, keys, None)
+        comp, edges = out
+        parts.append(edges)
+        n_comp -= int(edges[0].numel())                  # every recorded edge joins two components
+        if stats is not None:
+            stats["rounds"] += 1
+            stats["sweeps"] += int(swept)
+            stats["round_ms"].append((time.perf_counter() - t0) * 1e3)
+            stats["swept"].append(swept)
+    buf = sigT = None
+    u = torch.cat([p[0] for p in parts])
+    v = torch.cat([p[1] for p in parts])
+    bits = torch.cat([p[2] for p in parts])
+    order = torch.argsort(v, stable=True)                # (dist, u, v) by stable sorts, last key first
+    order = order[torch.argsort(u[order], stable=True)]
+    order = order[torch.argsort(bits[order], stable=True)]
+    return u[order].int(), v[order].int(), bits[order].view(torch.float32)
+
+
+def single_linkage_host(u: np.ndarray, v: np.ndarray, dist: np.ndarray, n: int) -> np.ndarray:
+    """scipy's linkage matrix Z float64[N-1, 4] from the MST edges sorted by dist (hsd_single_linkage_host):
+    row t merges the clusters holding u[t] and v[t] at height dist[t]; ids below N are nodes, N + s is the
+    cluster row s formed; Z[t, 0] < Z[t, 1] and Z[t, 3] is the new cluster's size."""
+    n = int(n)
+    u = np.ascontiguousarray(u, dtype=np.int32)
+    v = np.ascontiguousarray(v, dtype=np.int32)
+    dist = np.ascontiguousarray(dist, dtype=np.float32)
+    m = max(n - 1, 0)
+    if u.shape != (m,) or v.shape != (m,) or dist.shape != (m,):
+        raise ValueError(f"single_linkage_host: u, v and dist must hold n - 1 = {m} edges")
+    Z = np.zeros((m, 4), dtype=np.float64)
+    check(lib.hsd_single_linkage_host(u.ctypes.data, v.ctypes.data, dist.ctypes.data, n, Z.ctypes.data))
+    return Z
 
 
 def fp32_issue_peak(iters: int = 20000, reps: int = 3) -> float:

@@ -333,6 +333,32 @@ class HSD(object):
         return tuple(t.cpu().numpy() for t in out)
 
     @on_model_device
+    def minimum_spanning_tree(self, block_bytes=None):
+        """(u, v, dist): the minimum spanning tree of the complete graph over the nodes under the structural
+        distance (degree mode).  u < v are int32[N-1] node indices (model.nodes), dist float32[N-1], sorted by
+        (dist, u, v).  It is the unique MST under the order E(u, v) = (float(D[u, v]), u, v), D being the matrix
+        structural_distance_device holds: Kruskal in that order on D, bit for bit.  Built by Borůvka rounds over
+        row panels of at most ``block_bytes`` (as for nearest_neighbors; engine.degree_mst), so graphs whose
+        matrix exceeds the device memory work too."""
+        if self.signal != "degree":
+            raise NotImplementedError("minimum_spanning_tree is degree mode only (signal='degree')")
+        if self.n_node == 0:
+            return np.zeros(0, np.int32), np.zeros(0, np.int32), np.zeros(0, np.float32)
+        dg = self._device_graph(include_zero=(self.empty == "zero"))
+        out = engine.degree_mst(dg, self.hop, empty=self.empty, block_bytes=block_bytes)
+        return tuple(t.cpu().numpy() for t in out)
+
+    def single_linkage(self, block_bytes=None):
+        """Z float64[N-1, 4]: the single-linkage dendrogram in scipy's linkage format, which
+        scipy.cluster.hierarchy.fcluster and dendrogram take as is.  Row t merges clusters Z[t, 0] < Z[t, 1] at
+        height Z[t, 2], the t-th edge of minimum_spanning_tree, into a cluster of Z[t, 3] nodes; ids below N are
+        nodes (model.nodes), N + t is the cluster row t formed.  Where all pair distances differ, Z equals
+        scipy.cluster.hierarchy.linkage(squareform(D), "single").  Cutting it at height r
+        (fcluster(Z, r, "distance")) gives the connected components of radius_neighbors(r)."""
+        u, v, dist = self.minimum_spanning_tree(block_bytes=block_bytes)
+        return engine.single_linkage_host(u, v, dist, self.n_node)
+
+    @on_model_device
     def parallel_calculate_HSD(self, n_workers=3, row_signal="reference"):
         """model/HSD.py:118-137 with the worker of :140-161: hops 0..hop-1 of the zero-padded
         'aligned' distance (tools/metrics.py:151-192).  row_signal="reference" reproduces the

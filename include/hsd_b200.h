@@ -405,6 +405,33 @@ int hsd_radius_merge_parts(int32_t n_parts, int32_t n_rows, const int64_t* part_
                            const int32_t* idx, const void* val, int32_t elem_bytes, const int64_t* indptr,
                            int32_t* idx_out, void* val_out, void* stream);
 
+/* K7 minimum spanning tree: the MST of the complete graph under the distance, by Borůvka rounds over the
+ * same row panels (hsd_b200/engine.py::degree_mst), so the N x N matrix never has to exist.  Edges are
+ * ordered by E(u, v) = (D[u][v], min(u, v), max(u, v)); for a fixed node i that is the order of (D[i][j], j),
+ * so node i's best edge leaving its component is the minimum of the int64 key
+ * K(d, j) = float_bits(d) << 32 | j (distances finite and >= 0); INT64_MAX stands for "no edge".  comp
+ * int32[N] labels the components.  Keys are minima: results do not depend on the schedule.
+ *
+ * hsd_mst_panel_min: blk float[n_rows][ld] (n_rows <= n_cols <= ld) is a panel whose row r is node
+ *   node0 + r and whose column c is node node0 + c; only its upper part (c > r) is read.  For every element
+ *   with comp[a] != comp[b] (a = node0 + r, b = node0 + c) key_io[a] is lowered to K(blk[r][c], b) and
+ *   key_io[b] to K(blk[r][c], a); smaller keys already there are kept.
+ * hsd_mst_list_candidates: idx / val [n][k] (1 <= k <= 64) are k-NN lists ordered by (distance, id) and
+ *   padded with -1 / +inf (degree_knn's).  key_out[i] = K of the first entry of node i's list outside its
+ *   component, and bound_out[i] = +inf; when there is none, key_out[i] = INT64_MAX and bound_out[i] is the
+ *   distance of the k-th entry (every edge of i leaving its component is at least that long), or +inf when
+ *   the list is short (it holds every other node).
+ * hsd_single_linkage_host (HOST pointers, no CUDA): the n - 1 MST edges (u[t], v[t], dist[t]) in
+ *   non-decreasing dist -> Z double[n - 1][4] in scipy's linkage format: row t merges the clusters holding
+ *   u[t] and v[t], ids Z[t][0] < Z[t][1] (ids below n are nodes, n + s is the cluster row s formed), at height
+ *   dist[t], into a cluster of Z[t][3] nodes.  Edges that are not distinct nodes in 0..n-1, heights that are
+ *   not finite, negative or decreasing, and an edge that closes a cycle are rejected. */
+int hsd_mst_panel_min(const float* blk, int64_t ld, int32_t n_rows, int32_t n_cols, int32_t node0,
+                      const int32_t* comp, int64_t* key_io, void* stream);
+int hsd_mst_list_candidates(const int32_t* idx, const float* val, int32_t n, int32_t k, const int32_t* comp,
+                            int64_t* key_out, float* bound_out, void* stream);
+int hsd_single_linkage_host(const int32_t* u, const int32_t* v, const float* dist, int32_t n, double* Z);
+
 /* ---- e2e path: ship each unordered pair once, mirror on the host --------------------
  * The reference returns the dense symmetric ndarray (model/HSD.py:100-114, dist_mat[i,j] =
  * dist_mat[j,i]).  Over PCIe the matrix is the e2e bottleneck, so the host pipeline copies only
