@@ -539,9 +539,11 @@ def degree_knn(dg: DeviceGraph, hops: int, k: int, empty: str = "raise", block_b
     fits there is one panel, i.e. the launches of the resident path.
     panel_rows: force the panel height (a multiple of 128; tests).
     world > 1 with an initialised process group: every rank builds its dealt signatures (ShardedDegreeHSD),
-    sweeps its share of the panels (knn_deal) into its own lists, and one all-gather + hsd_topk_merge gives
-    every rank the whole result.  Without a process group the table is built on this device and this
-    rank's PARTIAL lists are returned (ranks emulated in one process; merge them with topk_merge).
+    the ranks agree on the panel height (MIN over the group: each rank's default comes from its own free
+    memory or block_bytes), each sweeps its share of the panels (knn_deal) into its own lists, and one
+    all-gather + hsd_topk_merge gives every rank the whole result.  Without a process group the table is
+    built on this device and this rank's PARTIAL lists are returned (ranks emulated in one process; merge
+    them with topk_merge).
     pair_events: a list that receives (r0, r1, start, end) per panel swept here, start / end being CUDA events
     around the panel's pairwise launches."""
     if empty not in ("raise", "zero"):
@@ -566,10 +568,14 @@ def _knn_sweep(sigT: torch.Tensor, dg: DeviceGraph, hops: int, k: int, block_byt
     dev = dg.rowptr.device
     k_used = dg.k_used(hops)
     if panel_rows is None:
-        if block_bytes is None:    # free memory, counting blocks torch's allocator holds but does not use
-            free = torch.cuda.mem_get_info(dev)[0] + torch.cuda.memory_reserved(dev) - torch.cuda.memory_allocated(dev)
-            block_bytes = int(free * KNN_BLOCK_FRACTION)
+        if block_bytes is None:
+            block_bytes = int(_free_bytes(dev) * KNN_BLOCK_FRACTION)
         panel_rows = knn_panel_rows(n, block_bytes, world)
+    if world > 1 and dist.is_available() and dist.is_initialized():
+        # a height taken from each rank's own free memory or block_bytes could differ: the ranks would deal
+        # different panel lists, and rows would be swept by no rank or by two
+        from .sharded import agree_min
+        panel_rows, = agree_min([panel_rows], group, dev)
     mine = knn_deal(n, knn_panels(n, panel_rows), world)[rank]
     idx = torch.full((n, k), -1, dtype=torch.int32, device=dev)
     val = torch.full((n, k), float("inf"), dtype=torch.float32, device=dev)
