@@ -23,6 +23,7 @@ HEADER_SYMBOLS = [
     "hsd_radius_count", "hsd_radius_emit_rows", "hsd_radius_emit_cols", "hsd_radius_scatter",
     "hsd_radius_merge_parts",
     "hsd_mst_panel_min", "hsd_mst_list_candidates", "hsd_single_linkage_host",
+    "hsd_mst_panel_min_mreach", "hsd_mst_list_candidates_mreach", "hsd_hdbscan_host",
 ]
 
 
@@ -92,6 +93,9 @@ lib.hsd_radius_merge_parts.argtypes = [c_int32, c_int32, _P, _P, _P, _P, c_int32
 lib.hsd_mst_panel_min.argtypes = [_P, c_int64, c_int32, c_int32, c_int32, _P, _P, _P]
 lib.hsd_mst_list_candidates.argtypes = [_P, _P, c_int32, c_int32, _P, _P, _P, _P]
 lib.hsd_single_linkage_host.argtypes = [_P, _P, _P, c_int32, _P]
+lib.hsd_mst_panel_min_mreach.argtypes = [_P, c_int64, c_int32, c_int32, c_int32, _P, _P, _P, _P]
+lib.hsd_mst_list_candidates_mreach.argtypes = [_P, _P, c_int32, c_int32, _P, _P, _P, _P, _P]
+lib.hsd_hdbscan_host.argtypes = [_P, c_int32, c_int32, c_int32, c_int32, _P, _P]
 lib.hsd_fp32_peak_probe.argtypes = [_P, c_int32, POINTER(c_int64), _P]
 lib.hsd_exact_wavelets.argtypes = [_P, c_int64, _P, c_int32, c_double, c_double, c_int32, _P, c_int64, _P]
 lib.hsd_copy2d_to_host.argtypes = [_P, c_int64, _P, c_int64, c_int64, c_int64, _P]

@@ -1001,16 +1001,54 @@ def degree_mst(dg: DeviceGraph, hops: int, empty: str = "raise", block_bytes: Op
     receives rounds, sweeps, the wall time in ms before round 1 (setup_ms: signatures and the lists; the device
     is synchronised there), per-round wall times (round_ms; a sweep round's includes its failed list try) and
     which rounds swept (swept)."""
-    import time
     if empty not in ("raise", "zero"):
         raise ValueError("empty must be 'raise' or 'zero'")
     if not 0 <= cand_k <= 64:
         raise ValueError("cand_k must be in 0..64")
+    return _boruvka(dg, hops, empty, block_bytes, cand_k, panel_rows, stats, 1)[:3]
+
+
+def degree_mreach_mst(dg: DeviceGraph, hops: int, min_samples: int, empty: str = "raise",
+                      block_bytes: Optional[int] = None, cand_k: int = MST_CAND_K, panel_rows: Optional[int] = None,
+                      stats: Optional[dict] = None) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
+    """The minimum spanning tree of HDBSCAN's mutual-reachability distance over the degree-mode distance D, without
+    the N x N matrix: (u int32[N-1], v int32[N-1], dist float32[N-1], core float32[N]).  core[i] is node i's core
+    distance, the (min_samples - 1)-th smallest D[i, j] over j != i (0 when min_samples = 1): scikit-learn's
+    np.partition(D, min_samples - 1, axis=1)[:, min_samples - 1], the zero diagonal counted ("min_samples includes
+    the point itself").  d_mr(i, j) = max(core[i], core[j], D[i, j]), one of its float32 operands exactly.  The tree
+    is the unique MST under E(u, v) = (d_mr(u, v), u, v): u < v, sorted by (dist, u, v), dist = d_mr — Kruskal in
+    that order on the dense d_mr, bit for bit.
+
+    degree_mst's Borůvka rounds over d_mr.  One k-NN sweep with k = max(cand_k, min_samples - 1) gives the cores
+    (val[:, min_samples - 2]) and, with cand_k > 0, the candidate lists.  The lists are ordered by D, not by d_mr,
+    so their keys (hsd_mst_list_candidates_mreach) certify less than degree_mst's and more rounds may sweep
+    (hsd_mst_panel_min_mreach).  min_samples = 1 is degree_mst (cores 0, its kernels).
+    min_samples: 1..65 (the top-k kernels take k <= 64) and at most N, else ValueError.  Other arguments and stats
+    as degree_mst's."""
+    if empty not in ("raise", "zero"):
+        raise ValueError("empty must be 'raise' or 'zero'")
+    if not 0 <= cand_k <= 64:
+        raise ValueError("cand_k must be in 0..64")
+    if not 1 <= min_samples <= 65:
+        raise ValueError(f"min_samples must be in 1..65 (got {min_samples})")
+    if min_samples > dg.n:
+        raise ValueError(f"min_samples ({min_samples}) must be at most the number of nodes ({dg.n})")
+    u, v, dist, core = _boruvka(dg, hops, empty, block_bytes, cand_k, panel_rows, stats, min_samples)
+    return u, v, dist, torch.zeros(dg.n, dtype=torch.float32, device=u.device) if core is None else core
+
+
+def _boruvka(dg: DeviceGraph, hops: int, empty: str, block_bytes: Optional[int], cand_k: int,
+             panel_rows: Optional[int], stats: Optional[dict], min_samples: int):
+    """The rounds of degree_mst (min_samples = 1) and degree_mreach_mst (min_samples > 1: keys on d_mr, from the
+    *_mreach kernels).  Arguments checked by the callers.  Returns (u, v, dist, core), core None when
+    min_samples = 1: degree_mst's launches are exactly those of the plain kernels."""
+    import time
     n = dg.n
     dev = dg.rowptr.device
     k_used = dg.k_used(hops)
+    core = None
     empty_out = (torch.zeros(0, dtype=torch.int32, device=dev), torch.zeros(0, dtype=torch.int32, device=dev),
-                 torch.zeros(0, dtype=torch.float32, device=dev))
+                 torch.zeros(0, dtype=torch.float32, device=dev), core)
     t_call = time.perf_counter()
     if stats is not None:
         stats.update(rounds=0, sweeps=0, round_ms=[], swept=[], setup_ms=0.0)
@@ -1021,8 +1059,12 @@ def degree_mst(dg: DeviceGraph, hops: int, empty: str = "raise", block_bytes: Op
         raise EmptyRingError("Distribution can't be empty.")
     if n < 2:
         return empty_out
-    if cand_k:
-        idx, val = _knn_sweep(sigT, dg, hops, cand_k, block_bytes, panel_rows)
+    list_k = max(cand_k, min_samples - 1)
+    mreach = min_samples > 1
+    if list_k:
+        idx, val = _knn_sweep(sigT, dg, hops, list_k, block_bytes, panel_rows)
+        if mreach:
+            core = val[:, min_samples - 2].contiguous()
     if stats is not None:                                # the lists' sweep is not part of round 1
         torch.cuda.synchronize(dev)
         stats["setup_ms"] = (time.perf_counter() - t_call) * 1e3
@@ -1035,8 +1077,12 @@ def degree_mst(dg: DeviceGraph, hops: int, empty: str = "raise", block_bytes: Op
         t0 = time.perf_counter()
         out = None
         if cand_k:
-            check(lib.hsd_mst_list_candidates(_ptr(idx), _ptr(val), n, cand_k, _ptr(comp), _ptr(keys), _ptr(bound),
-                                              st))
+            if mreach:
+                check(lib.hsd_mst_list_candidates_mreach(_ptr(idx), _ptr(val), n, list_k, _ptr(comp), _ptr(core),
+                                                         _ptr(keys), _ptr(bound), st))
+            else:
+                check(lib.hsd_mst_list_candidates(_ptr(idx), _ptr(val), n, cand_k, _ptr(comp), _ptr(keys),
+                                                  _ptr(bound), st))
             out = _mst_contract(comp, keys, bound)
         swept = out is None
         if swept:
@@ -1056,7 +1102,11 @@ def degree_mst(dg: DeviceGraph, hops: int, empty: str = "raise", block_bytes: Op
                 R, ld = r1 - r0, roundup(n - r0, 4)
                 B = buf[:R * ld].view(R, ld)
                 _panel_pairwise(sigT, k_used, n, r0, r1, B, ld, st)
-                check(lib.hsd_mst_panel_min(B.data_ptr(), ld, R, n - r0, r0, _ptr(comp), _ptr(keys), st))
+                if mreach:
+                    check(lib.hsd_mst_panel_min_mreach(B.data_ptr(), ld, R, n - r0, r0, _ptr(comp), _ptr(core),
+                                                       _ptr(keys), st))
+                else:
+                    check(lib.hsd_mst_panel_min(B.data_ptr(), ld, R, n - r0, r0, _ptr(comp), _ptr(keys), st))
             out = _mst_contract(comp, keys, None)
         comp, edges = out
         parts.append(edges)
@@ -1073,7 +1123,7 @@ def degree_mst(dg: DeviceGraph, hops: int, empty: str = "raise", block_bytes: Op
     order = torch.argsort(v, stable=True)                # (dist, u, v) by stable sorts, last key first
     order = order[torch.argsort(u[order], stable=True)]
     order = order[torch.argsort(bits[order], stable=True)]
-    return u[order].int(), v[order].int(), bits[order].view(torch.float32)
+    return u[order].int(), v[order].int(), bits[order].view(torch.float32), core
 
 
 def single_linkage_host(u: np.ndarray, v: np.ndarray, dist: np.ndarray, n: int) -> np.ndarray:
@@ -1090,6 +1140,28 @@ def single_linkage_host(u: np.ndarray, v: np.ndarray, dist: np.ndarray, n: int) 
     Z = np.zeros((m, 4), dtype=np.float64)
     check(lib.hsd_single_linkage_host(u.ctypes.data, v.ctypes.data, dist.ctypes.data, n, Z.ctypes.data))
     return Z
+
+
+HDBSCAN_METHODS = {"eom": 0, "leaf": 1}
+
+
+def hdbscan_host(Z: np.ndarray, n: int, min_cluster_size: int, method: str = "eom",
+                 allow_single_cluster: bool = False) -> Tuple[np.ndarray, np.ndarray]:
+    """(labels int64[N], probabilities float64[N]) of HDBSCAN from the single-linkage tree Z (single_linkage_host's,
+    float64[N-1, 4]) of the mutual-reachability MST (hsd_hdbscan_host): scikit-learn's
+    tree_to_labels(Z, min_cluster_size, method, allow_single_cluster, 0.0, None), bit for bit.  -1 is noise.
+    N >= 2, min_cluster_size >= 2, method "eom" or "leaf"."""
+    if method not in HDBSCAN_METHODS:
+        raise ValueError(f"cluster_selection_method must be 'eom' or 'leaf' (got {method!r})")
+    n = int(n)
+    Z = np.ascontiguousarray(Z, dtype=np.float64)
+    if Z.shape != (max(n - 1, 0), 4):
+        raise ValueError(f"hdbscan_host: Z must be float64[n - 1, 4] (n = {n})")
+    labels = np.empty(max(n, 0), dtype=np.int64)
+    prob = np.empty(max(n, 0), dtype=np.float64)
+    check(lib.hsd_hdbscan_host(Z.ctypes.data, n, int(min_cluster_size), HDBSCAN_METHODS[method],
+                               int(bool(allow_single_cluster)), labels.ctypes.data, prob.ctypes.data))
+    return labels, prob
 
 
 def fp32_issue_peak(iters: int = 20000, reps: int = 3) -> float:

@@ -359,6 +359,58 @@ class HSD(object):
         return engine.single_linkage_host(u, v, dist, self.n_node)
 
     @on_model_device
+    def mutual_reachability_mst(self, min_samples=5, block_bytes=None):
+        """(u, v, dist): the minimum spanning tree of HDBSCAN's mutual-reachability distance (degree mode), the tree
+        hdbscan labels.  core(i) is the (min_samples - 1)-th smallest D[i, j] over j != i, 0 when min_samples = 1
+        (scikit-learn's convention: min_samples includes the point itself), and d_mr(i, j) = max(core(i), core(j),
+        D[i, j]), D being the matrix structural_distance_device holds.  u < v are int32[N-1] node indices
+        (model.nodes), dist = d_mr float32[N-1], sorted by (dist, u, v): the unique MST under the order
+        E(u, v) = (d_mr(u, v), u, v), Kruskal in that order on the dense d_mr, bit for bit.  Built without the
+        N x N matrix (engine.degree_mreach_mst), in row panels of at most ``block_bytes`` as for
+        nearest_neighbors.  min_samples: 1..65 and at most N, else ValueError."""
+        if self.signal != "degree":
+            raise NotImplementedError("mutual_reachability_mst is degree mode only (signal='degree')")
+        dg = self._device_graph(include_zero=(self.empty == "zero"))
+        out = engine.degree_mreach_mst(dg, self.hop, min_samples, empty=self.empty, block_bytes=block_bytes)
+        return tuple(t.cpu().numpy() for t in out[:3])
+
+    def hdbscan(self, min_cluster_size=5, min_samples=None, cluster_selection_method="eom",
+                allow_single_cluster=False, block_bytes=None):
+        """(labels int64[N], probabilities float64[N]): HDBSCAN of the structural distance (degree mode), what
+        sklearn.cluster.HDBSCAN(metric="precomputed", ...).fit(D) computes, without the N x N matrix.  labels are
+        cluster ids 0, 1, ... over node indices (model.nodes), -1 for noise; probabilities are the membership
+        strengths (0 for noise).  min_samples=None means min_cluster_size, as in scikit-learn.
+
+        The labels are scikit-learn's tree_to_labels(Z, min_cluster_size, cluster_selection_method,
+        allow_single_cluster, 0.0, None) bit for bit, Z being single_linkage_host's linkage of
+        mutual_reachability_mst(min_samples) (engine.hdbscan_host).  Ties: when several spanning trees are minimal
+        (many pairs at distance 0, many edges at some node's core distance), HDBSCAN's output depends on the one
+        chosen.  This one takes the unique tree under E = (d_mr, u, v), so the output is well defined;
+        scikit-learn's fit chooses among tied trees by Prim's order and an unstable sort, and matches it where the
+        tree's heights are pairwise distinct.  The sorted heights are the same for every minimal tree.
+        ValueError, as scikit-learn's: N < 2, min_samples > N, min_cluster_size < 2, an unknown
+        cluster_selection_method; also min_samples > 65.  NotImplementedError in wavelet mode.  Empty rings follow
+        model.empty, as in the other degree-mode methods."""
+        if int(min_cluster_size) != min_cluster_size or min_cluster_size < 2:
+            raise ValueError(f"min_cluster_size must be an integer >= 2 (got {min_cluster_size!r})")
+        if min_samples is None:
+            min_samples = min_cluster_size
+        if int(min_samples) != min_samples or min_samples < 1:
+            raise ValueError(f"min_samples must be None or an integer >= 1 (got {min_samples!r})")
+        if cluster_selection_method not in engine.HDBSCAN_METHODS:
+            raise ValueError(f"cluster_selection_method must be 'eom' or 'leaf' (got {cluster_selection_method!r})")
+        if self.signal != "degree":
+            raise NotImplementedError("hdbscan is degree mode only (signal='degree')")
+        n = self.n_node
+        if n < 2:
+            raise ValueError(f"n_samples={n} while HDBSCAN requires more than one sample")
+        if min_samples > n:
+            raise ValueError(f"min_samples ({min_samples}) must be at most the number of samples ({n})")
+        u, v, dist = self.mutual_reachability_mst(int(min_samples), block_bytes=block_bytes)
+        Z = engine.single_linkage_host(u, v, dist, n)
+        return engine.hdbscan_host(Z, n, int(min_cluster_size), cluster_selection_method, allow_single_cluster)
+
+    @on_model_device
     def parallel_calculate_HSD(self, n_workers=3, row_signal="reference"):
         """model/HSD.py:118-137 with the worker of :140-161: hops 0..hop-1 of the zero-padded
         'aligned' distance (tools/metrics.py:151-192).  row_signal="reference" reproduces the

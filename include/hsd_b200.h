@@ -432,6 +432,28 @@ int hsd_mst_list_candidates(const int32_t* idx, const float* val, int32_t n, int
                             int64_t* key_out, float* bound_out, void* stream);
 int hsd_single_linkage_host(const int32_t* u, const int32_t* v, const float* dist, int32_t n, double* Z);
 
+/* K7b mutual-reachability minimum spanning tree (HDBSCAN; hsd_b200/engine.py::degree_mreach_mst): the MST above
+ * under d_mr(a, b) = max(core[a], core[b], D[a][b]), core float[N] finite and >= 0 (node i's core distance), so
+ * d_mr is one of its operands and keys are K(d_mr, j).
+ *
+ * hsd_mst_panel_min_mreach: hsd_mst_panel_min with the compared value max(blk[r][c], core[a], core[b]).
+ * hsd_mst_list_candidates_mreach: the lists are ordered by D, not by d_mr.  key_out[i] = the minimum of
+ *   K(max(core[i], core[j], val[i][t]), j) over the entries j of node i's list outside its component
+ *   (INT64_MAX when there is none).  bound_out[i] = +inf when that key is exact: the list is short (it holds
+ *   every other node) or the key's distance is strictly below val[i][k-1] (an unlisted j has
+ *   d_mr(i, j) >= D[i][j] >= val[i][k-1]); else bound_out[i] = val[i][k-1], a lower bound of every unlisted
+ *   edge of i.
+ * hsd_hdbscan_host (HOST pointers, no CUDA): Z double[n - 1][4], hsd_single_linkage_host's linkage of the
+ *   mutual-reachability MST -> labels int64[n] (-1: noise) and probabilities double[n], what scikit-learn's
+ *   HDBSCAN tree_to_labels(Z, min_cluster_size, method, allow_single_cluster, 0.0, None) returns, with the
+ *   same float64 operations in the same order.  method 0 = "eom", 1 = "leaf"; n >= 2, min_cluster_size >= 2. */
+int hsd_mst_panel_min_mreach(const float* blk, int64_t ld, int32_t n_rows, int32_t n_cols, int32_t node0,
+                             const int32_t* comp, const float* core, int64_t* key_io, void* stream);
+int hsd_mst_list_candidates_mreach(const int32_t* idx, const float* val, int32_t n, int32_t k, const int32_t* comp,
+                                   const float* core, int64_t* key_out, float* bound_out, void* stream);
+int hsd_hdbscan_host(const double* Z, int32_t n, int32_t min_cluster_size, int32_t method,
+                     int32_t allow_single_cluster, int64_t* labels, double* probabilities);
+
 /* ---- e2e path: ship each unordered pair once, mirror on the host --------------------
  * The reference returns the dense symmetric ndarray (model/HSD.py:100-114, dist_mat[i,j] =
  * dist_mat[j,i]).  Over PCIe the matrix is the e2e bottleneck, so the host pipeline copies only
